@@ -46,6 +46,7 @@ CHR1 = 248956422
 WINDOW_SIZE, WINDOW_SHIFT, CONSTRAINT = 2500, 1250, 'constants'
 FP64_OPS_PER_CELL = 4            # DMUL s*Lg, DADD G-.., DADD +P_i, compare (SURVEY 8d)
 BIG_CONTIG = 16 << 20            # genome leg: shorter contigs share one batched launch sequence
+DUMP_MAX_SEGMENTS = 1 << 20      # --dump-outputs: five float64 arrays of at most this length, 40 MB in all
 
 
 def measured_peaks():
@@ -359,6 +360,23 @@ def exact_leg(eng, peak_nominal):
     return out
 
 
+def dump_outputs(out_dir, splits, scores, means, total_score):
+    """The segmentation of the last timed step as float64 .npy files under out_dir, for comparing two builds output for
+    output: per segment its index, start, stop, score and mean count, for every segment when there are at most
+    DUMP_MAX_SEGMENTS of them and otherwise for a fixed seeded sample of that many; plus the total score and the number
+    of segments.  float64 holds every position and index exactly."""
+    nseg = len(splits) - 1
+    idx = np.arange(nseg)
+    if nseg > DUMP_MAX_SEGMENTS:
+        idx = np.sort(np.random.RandomState(0).choice(nseg, DUMP_MAX_SEGMENTS, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {'segment_index': idx, 'segment_start': splits[idx], 'segment_stop': splits[idx + 1],
+              'segment_score': scores[idx], 'segment_mean': means[idx],
+              'total_score': [total_score], 'n_segments': [nseg]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), np.asarray(a, dtype=np.float64))
+
+
 # ------------------------------------------------------------------------------------------------
 def run_b200(args):
     genome_host = genome_generate(args)          # host data of this rank's LPT share, before CUDA starts (fork pool)
@@ -392,8 +410,8 @@ def run_b200(args):
         eng.load_device(resident.data_ptr(), n, owner=resident)
         eng.set_candidates(None)
         _run_device_pipeline(eng, plan)
-        eng.segment_scores(scores=True, means=True)
-        return eng.candidate_count(), float(eng.segment_scores_sum())
+        scores, _, means, _ = eng.segment_scores(scores=True, means=True)
+        return eng.candidate_count(), float(eng.segment_scores_sum()), scores, means
 
     def step_e2e():
         eng.invalidate()                                     # force the H2D copy every step
@@ -402,7 +420,7 @@ def run_b200(args):
 
     # ---- device-resident throughput ------------------------------------------------------------
     for _ in range(args.warmup):
-        m_final, score = step_resident()
+        m_final, score = step_resident()[:2]
     fp64_peak_measured = eng.fp64_peak() if rank == 0 else 0.0
     eng.timing_reset(True)
     sampler = ClockSampler(local, str(getattr(torch.cuda.get_device_properties(local), 'uuid', '') or ''))
@@ -412,7 +430,8 @@ def run_b200(args):
     ev0.record(stream)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        m_final, score = step_resident()
+        last = None              # frees the previous step's pinned result buffers for this step to reuse
+        last = step_resident()
     ev1.record(stream)
     ev1.synchronize()
     wall = time.perf_counter() - t0
@@ -421,6 +440,10 @@ def run_b200(args):
     dev_ms = ev0.elapsed_time(ev1)
     timing = eng.timing()
     eng.timing_reset(False)
+    m_final, score = last[:2]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, eng.candidates(), last[2], last[3], score)
+    del last
     rank_rows = gather_rows([dev_ms / args.steps], dist, device, world)
     step_ms = max(r[0] for r in rank_rows)
     total_nt = float(n) * world
@@ -659,7 +682,13 @@ def main():
                     help='scale of the hg38 contig-size profile of the `genome` leg (configs[3]); 0 skips the leg')
     ap.add_argument('--genome-steps', type=int, default=2)
     ap.add_argument('--skip-exact', action='store_true', help='skip the `exact_dp` leg (configs[0], configs[2])')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write the segments of the last one as DIR/<name>.npy (float64)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes what the GPU path computed; --impl reference has no such output')
     if args.impl == 'reference':
         run_reference(args)
     else:
