@@ -174,6 +174,20 @@ int pasio_set_tuning(pasio_ctx *ctx, int key, int value);
 int pasio_rounds(pasio_ctx *ctx, int64_t window_size, int64_t window_shift, int constraint,
                  int64_t max_rounds, int64_t *rounds_done, int64_t *n_out, int64_t *cells,
                  int64_t *sizes, int64_t sizes_cap);
+/* Penalties of the window DP: while a term is set, pasio_round, pasio_rounds and pasio_contig_load_round run every
+ * window through SquareSplitter.split_with_normalizations (square_splitter.py:29-65, reached from
+ * sliding_window_reducer.py:10-18 when the window's base splitter is regularised) instead of
+ * split_without_normalizations; per cell, in that order,
+ *   t = self_score + P_i - split_number_penalty[num_splits_i] (+ first_column_refund for i = 0) - length_penalty[L_j - L_i],
+ * first arg-max, num_splits_j = prev_j ? num_splits[prev_j] + 1 : 0, positions and split numbers local to the window.
+ * The tables are those of pasio_square_split_regularized (square_splitter.py:46-54): split_number_penalty[k] =
+ * multiplier * function(k + 1), at least as many entries as the largest window has candidates (PASIO_E_ARG otherwise);
+ * length_penalty[len] = multiplier * function(len), as long as the log table (a round that needs more returns
+ * PASIO_E_TABLE_TOO_SHORT with pasio_table_need's log entry); first_column_refund = multiplier * function(1).  NULL
+ * switches a term off, both NULL clear the penalties; after an error both terms are off.  The tables are copied; pasio_square_split, the exact DP
+ * with its own tables and the scoring entry points do not use them. */
+int pasio_set_penalties(pasio_ctx *ctx, const double *split_number_penalty, int64_t n_split_number_penalty,
+                        double first_column_refund, const double *length_penalty, int64_t n_length_penalty);
 
 /* ---- exact DP -----------------------------------------------------------------------
  * Replaces SquareSplitter.split_without_normalizations + collect_split_points

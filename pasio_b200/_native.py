@@ -52,6 +52,7 @@ SIGNATURES = {
     'pasio_upload_stats': (ctypes.c_int, [_vp, _i64p]),
     'pasio_set_tuning': (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int]),
     'pasio_rounds': (ctypes.c_int, [_vp, _i64, _i64, ctypes.c_int, _i64, _i64p, _i64p, _i64p, _i64p, _i64]),
+    'pasio_set_penalties': (ctypes.c_int, [_vp, _f64p, _i64, ctypes.c_double, _f64p, _i64]),
     'pasio_square_split': (ctypes.c_int, [_vp, _i64p, _i64, _i64p, _f64p, _f64p, _i64p]),
     'pasio_square_split_regularized': (ctypes.c_int, [_vp, _f64p, _i64, _f64p, _i64, ctypes.c_double, _i64p, _i64, _i64p, _f64p,
                                                      _f64p, _i64p]),
@@ -165,6 +166,9 @@ class Engine(object):
         self._params = None          # (alpha_is_int, alpha, beta, pen)
         self._tables = {}            # table id -> (computer object, uploaded length)
         self._scorer_source = None   # object providing the three computers
+        self._penalty_spec = None    # penalty spec of the last use_scorer: what the next round applies
+        self._penalties = None       # (penalty spec, length of the length table) set on the device, or None
+        self._penalty_host = None    # (the same key, the host tables built for it): setting them again is an upload only
         self._loaded = None          # strong ref to the loaded counts array (identity cache)
         self._loaded_print = None    # its sampled content fingerprint
         self._cands_print = None
@@ -191,9 +195,13 @@ class Engine(object):
         raise PasioDeviceError('pasio_b200 error %d: %s' % (rc, msg))
 
     # -- scorer parameters and tables --------------------------------------------------------
-    def use_scorer(self, source):
+    def use_scorer(self, source, penalties=None):
         """source has .alpha (int or float), .beta, .log_computer, .log_gamma_computer,
-        .log_gamma_alpha_computer, .segment_creation_cost (ScorerFactory or a scorer)."""
+        .log_gamma_alpha_computer, .segment_creation_cost (ScorerFactory or a scorer).
+        penalties: the penalty_spec (splitters/square_splitter.py) of a regularised window splitter, which the rounds
+        then apply, or None; set or cleared on every call, so no later call inherits them.  Only the rounds read the
+        penalties, so the device follows this setting when the next round starts (_sync_penalties): switching them off
+        for scoring and on again for the next contig uploads nothing."""
         alpha = source.alpha
         is_int = isinstance(alpha, (int, np.integer)) and not isinstance(alpha, bool)
         params = (int(is_int), float(alpha), float(source.log_computer.shift), float(source.segment_creation_cost))
@@ -207,6 +215,29 @@ class Engine(object):
             if have is None or have[0] is not comp:
                 self._upload_table(tid, comp, comp.cache_size)
         self._scorer_source = source
+        self._penalty_spec = penalties
+
+    def _sync_penalties(self):
+        """Before a round: the device's penalty tables (pasio_set_penalties) are those of the last use_scorer.  The
+        split-number table covers the largest fused window, the length table is as long as the log table (both are
+        indexed by span)."""
+        spec = self._penalty_spec
+        want = None if spec is None else (spec, self._tables[TAB_LOG][1])
+        if want == self._penalties:
+            return
+        self._penalties = None       # pasio_set_penalties switches both terms off first: so does this record
+        if spec is None:
+            self._check(self.lib.pasio_set_penalties(self.ctx, None, 0, 0.0, None, 0))
+        else:
+            from .splitters.square_splitter import penalty_tables
+            from .splitters._fusion import MAX_FUSED_WINDOW_CANDIDATES
+            if self._penalty_host is None or self._penalty_host[0] != want:      # (a long length table costs seconds to build)
+                self._penalty_host = (want, penalty_tables(spec, want[1], MAX_FUSED_WINDOW_CANDIDATES))
+            lp, sp, refund = self._penalty_host[1]
+            self._check(self.lib.pasio_set_penalties(
+                self.ctx, None if sp is None else _ptr(sp, ctypes.c_double), 0 if sp is None else len(sp), refund,
+                None if lp is None else _ptr(lp, ctypes.c_double), 0 if lp is None else len(lp)))
+        self._penalties = want
 
     def _upload_table(self, tid, comp, n):
         tab = comp.table(n)
@@ -220,6 +251,8 @@ class Engine(object):
             comp, have = self._tables[tid]
             if need[tid].value > have:
                 self._upload_table(tid, comp, max(need[tid].value, int(have * 1.5)))
+        if self._penalty_spec is not None:
+            self._sync_penalties()                      # the length table follows the log table
 
     def _retry(self, fn):
         """Call fn() until it stops asking for longer tables."""
@@ -276,6 +309,7 @@ class Engine(object):
         self._cands_obj = None
         n_in, n_out, cells = _i64(0), _i64(0), _i64(0)
         self.set_tuning('logfac_eager', 1 if want_logfac else 0)
+        self._sync_penalties()
         try:
             rc = self.lib.pasio_contig_load_round(self.ctx, _ptr(c, ctypes.c_int64), len(c), window_size, window_shift,
                                                   CONSTRAINTS[constraint], ctypes.byref(n_in), ctypes.byref(n_out),
@@ -380,6 +414,7 @@ class Engine(object):
     def round(self, window_size, window_shift, constraint):
         n_in, n_out, cells = _i64(0), _i64(0), _i64(0)
         self._cands_obj = None
+        self._sync_penalties()
         self._retry(lambda: self.lib.pasio_round(self.ctx, window_size, window_shift, CONSTRAINTS[constraint],
                                                  ctypes.byref(n_in), ctypes.byref(n_out), ctypes.byref(cells)))
         return n_in.value, n_out.value, cells.value
@@ -417,6 +452,7 @@ class Engine(object):
             done, n_out, cells = _i64(0), _i64(0), _i64(0)
             buf = np.zeros(64, dtype=np.int64)
             step = min(limit, 64)
+            self._sync_penalties()
             rc = self.lib.pasio_rounds(self.ctx, window_size, window_shift, CONSTRAINTS[constraint], step,
                                        ctypes.byref(done), ctypes.byref(n_out), ctypes.byref(cells),
                                        _ptr(buf, ctypes.c_int64), len(buf))

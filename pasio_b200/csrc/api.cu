@@ -535,8 +535,11 @@ extern "C" int pasio_table_need(const pasio_ctx *ctx, int64_t *n_log, int64_t *n
     return PASIO_OK;
 }
 
-// DP tables must cover span (log) and count (+alpha for integer alpha)
-static int check_dp_tables(pasio_ctx *ctx, i64 max_span, i64 max_cnt)
+static bool penalties_on(const pasio_ctx *ctx) { return ctx->pen_num || ctx->pen_len; }
+
+// DP tables must cover span (log) and count (+alpha for integer alpha); with_penalties (the rounds): the length penalty
+// table is indexed by span exactly like the log table
+static int check_dp_tables(pasio_ctx *ctx, i64 max_span, i64 max_cnt, bool with_penalties = false)
 {
     if (!ctx->have_params) return pasio_fail(ctx, PASIO_E_STATE, "pasio_set_params has not been called");
     if (max_cnt + ctx->alpha_int >= 2147483647LL)
@@ -547,10 +550,35 @@ static int check_dp_tables(pasio_ctx *ctx, i64 max_span, i64 max_cnt)
     bool bad = false;
     if (ctx->ntab[PASIO_TAB_LOG] < need_log) { ctx->need[PASIO_TAB_LOG] = need_log; bad = true; }
     if (ctx->ntab[gid] < need_g) { ctx->need[gid] = need_g; bad = true; }
+    if (with_penalties && ctx->pen_len && ctx->n_pen_lr < need_log) { ctx->need[PASIO_TAB_LOG] = need_log; bad = true; }
     if (bad)
-        return pasio_fail(ctx, PASIO_E_TABLE_TOO_SHORT, "tables too short: need log>=%lld, lgamma[%d]>=%lld (have %lld, %lld)",
+        return pasio_fail(ctx, PASIO_E_TABLE_TOO_SHORT, "tables too short: need log>=%lld, lgamma[%d]>=%lld (have %lld, %lld%s)",
                           (long long)need_log, gid, (long long)need_g, (long long)ctx->ntab[PASIO_TAB_LOG],
-                          (long long)ctx->ntab[gid]);
+                          (long long)ctx->ntab[gid], with_penalties && ctx->pen_len ? ", length penalty as long as log" : "");
+    return PASIO_OK;
+}
+
+extern "C" int pasio_set_penalties(pasio_ctx *ctx, const double *split_number_penalty, int64_t n_split_number_penalty,
+                                   double first_column_refund, const double *length_penalty, int64_t n_length_penalty)
+{
+    NEED_CTX(ctx);
+    if ((split_number_penalty && n_split_number_penalty < 1) || (length_penalty && n_length_penalty < 1))
+        return pasio_fail(ctx, PASIO_E_ARG, "a penalty table needs at least one entry");
+    ctx->pen_num = ctx->pen_len = false;
+    if (split_number_penalty) {
+        PASIO_TRY(pasio_reserve(ctx, ctx->penNR, (size_t)n_split_number_penalty * 8));
+        PASIO_TRY(h2d(ctx, ctx->penNR.p, split_number_penalty, (size_t)n_split_number_penalty * 8));
+    }
+    if (length_penalty) {
+        PASIO_TRY(pasio_reserve(ctx, ctx->penLR, (size_t)n_length_penalty * 8));
+        PASIO_TRY(h2d(ctx, ctx->penLR.p, length_penalty, (size_t)n_length_penalty * 8));
+    }
+    CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));      // the caller's tables were read by the copies above
+    ctx->pen_num = split_number_penalty != nullptr;
+    ctx->n_pen_nr = ctx->pen_num ? n_split_number_penalty : 0;
+    ctx->pen_refund = ctx->pen_num ? first_column_refund : 0.0;
+    ctx->pen_len = length_penalty != nullptr;
+    ctx->n_pen_lr = ctx->pen_len ? n_length_penalty : 0;
     return PASIO_OK;
 }
 
@@ -814,10 +842,13 @@ extern "C" int pasio_contig_load_round(pasio_ctx *ctx, const int64_t *counts, in
                 cudaStreamSynchronize(ctx->stream_copy);      // the caller's buffer must not be read after we return
                 return pasio_fail(ctx, PASIO_E_COUNTS, "counts must be >= 0");
             }
-            table_rc = check_dp_tables(ctx, max_span, max_cnt);
+            table_rc = check_dp_tables(ctx, max_span, max_cnt, true);
             if (table_rc == PASIO_OK) {
-                PASIO_TRY(launch_window_dp(ctx, w_ready - w_done, (int)window_size, (int)window_shift, constraint, w_done,
-                                           !first_dp));
+                if (penalties_on(ctx))
+                    PASIO_TRY(launch_window_dp_reg(ctx, w_ready - w_done, (int)window_size, (int)window_shift, constraint, !first_dp));
+                else
+                    PASIO_TRY(launch_window_dp(ctx, w_ready - w_done, (int)window_size, (int)window_shift, constraint, w_done,
+                                               !first_dp));
                 first_dp = false;
             } else if (table_rc != PASIO_E_TABLE_TOO_SHORT) {
                 return table_rc;
@@ -1059,11 +1090,12 @@ extern "C" int pasio_round(pasio_ctx *ctx, int64_t window_size, int64_t window_s
                           "contig total %lld / length %lld (m=%lld, implicit=%d, windows=%lld)", (long long)max_cnt,
                           (long long)max_span, (long long)ctx->total, (long long)ctx->n, (long long)ctx->m,
                           (int)ctx->implicit_all, (long long)nwin);
-    PASIO_TRY(check_dp_tables(ctx, max_span, max_cnt));
+    PASIO_TRY(check_dp_tables(ctx, max_span, max_cnt, true));
 
     const size_t bit_bytes = (size_t)((ctx->n + 1 + 31) / 32 + 2) * 4;
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->keepbits.p, 0, bit_bytes, ctx->stream));
-    PASIO_TRY(launch_window_dp(ctx, nwin, (int)window_size, (int)window_shift, constraint));
+    if (penalties_on(ctx)) PASIO_TRY(launch_window_dp_reg(ctx, nwin, (int)window_size, (int)window_shift, constraint));
+    else PASIO_TRY(launch_window_dp(ctx, nwin, (int)window_size, (int)window_shift, constraint));
 
     // survivors: at most the current count (the new list is a subset, round_reducer.py:25)
     const int nxt = 1 - ctx->cur;

@@ -97,6 +97,12 @@ struct pasio_ctx {
     // scratch
     DevBuf blocksum, tilestate, scalars, dpL, dpC, dpP, dpPrev, dpPart, dpPartArg, dpMark, dpJump, fscan, logfac_full;
     DevBuf xpRing, xpRec, xpTasks, regLR, regNR;
+
+    // penalties of the rounds (pasio_set_penalties): NR[k] split-number, LR[len] length table, first-column refund
+    bool pen_num = false, pen_len = false;
+    DevBuf penNR, penLR;
+    i64 n_pen_nr = 0, n_pen_lr = 0;
+    double pen_refund = 0.0;
     DevBuf lxPos, lxSum, lxFirst, lxState;    // logfac_exact.cu: positions / running sums of the non-zero log-factorial terms, first term per contig
     i64 lx_terms = 0;
     i64 scan_tiles_done = 0;     // tiles of the loaded contig already scanned (pasio_contig_load_round scans chunk by chunk)   // exact_pruned.cu: self-score ring, column-block records, task list
@@ -159,6 +165,9 @@ int launch_boundary_ranks(pasio_ctx *ctx);                    // brank from curr
 // classify_constraint >= 0: also sort the windows into ctx->win_small / win_large (n_small, n_large) for launch_window_dp
 int launch_window_prepass(pasio_ctx *ctx, i64 nwin, int wsize, int wshift, i64 *h_max_span, i64 *h_max_cnt,
                           int classify_constraint = -1, i64 w_begin = 0);  // windows [w_begin, w_begin + nwin); syncs
+// most candidates the warp-per-window kernels take (small / medium class), shared by K4 (window_dp.cu) and K8
+// (window_dp_reg.cu) because the prepass sorts the windows for both
+constexpr int WD_SMALL_MAX_CANDIDATES = 160, WD_MEDIUM_MAX_CANDIDATES = 512;
 int small_window_max_candidates();                           // window_dp.cu: most candidates the warp-per-window kernels take
 int medium_window_max_candidates();
 int launch_validate_candidates(pasio_ctx *ctx, i64 *h_bad);   // syncs
@@ -168,6 +177,10 @@ int launch_filter_candidates(pasio_ctx *ctx, int constraint);  // current candid
 int launch_window_dp(pasio_ctx *ctx, i64 nwin, int wsize, int wshift, int constraint, i64 w_begin = 0,
                      bool keep_cell_counters = false);   // windows [w_begin, w_begin + nwin)
 int window_dp_max_candidates(pasio_ctx *ctx);
+
+// window_dp_reg.cu: the same round with the penalties of pasio_set_penalties (needs the classified prepass lists)
+int launch_window_dp_reg(pasio_ctx *ctx, i64 nwin, int wsize, int wshift, int constraint, bool keep_cell_counters = false);
+int window_dp_reg_max_candidates(pasio_ctx *ctx);
 
 // exact_dp.cu
 int launch_exact_dp(pasio_ctx *ctx, i64 N);                   // over ctx->dpL/dpC -> dpP/dpPrev

@@ -760,8 +760,8 @@ window_dp_kernel(WinDpParams p)
 // sweeps every second finished column for its row, the 16 x 16 triangle is resolved in order by shuffles.
 // Two size classes: up to 160 candidates (8 windows per CTA, 5 CTAs per SM) and up to 512 (4 per CTA, 4 CTAs per SM).
 constexpr int SW_JB = 16;
-constexpr int SW_SMALL_N = 160, SW_SMALL_WARPS = 8, SW_SMALL_CTAS = 5;
-constexpr int SW_MEDIUM_N = 512, SW_MEDIUM_WARPS = 4, SW_MEDIUM_CTAS = 4;
+constexpr int SW_SMALL_N = WD_SMALL_MAX_CANDIDATES, SW_SMALL_WARPS = 8, SW_SMALL_CTAS = 5;
+constexpr int SW_MEDIUM_N = WD_MEDIUM_MAX_CANDIDATES, SW_MEDIUM_WARPS = 4, SW_MEDIUM_CTAS = 4;
 
 template <int MAXN>
 struct __align__(16) SmallWin {

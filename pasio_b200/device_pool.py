@@ -32,7 +32,7 @@ def _worker(device, jobs, shm_name, n_runs, splitter_blob, mode, tmpdir, done_q)
         from . import process_bedgraph
         from .splitters import _fusion
         splitter = pickle.loads(splitter_blob)
-        plan = _fusion.pipeline_plan(splitter)
+        plan = _fusion.device_plan(splitter)
         shm, runs = _attach(shm_name, n_runs)
         try:
             for index, contigs in jobs:

@@ -375,7 +375,7 @@ def split_bedgraph_stream(input_stream, output_stream, splitter, split_at_gaps=F
     that many GPUs by longest-processing-time-first, one worker process per GPU, the text gathered on the host in
     input order (device_pool.py)."""
     logger.info('Reading input file')
-    plan = _fusion.pipeline_plan(splitter)
+    plan = _fusion.device_plan(splitter)
     if output_mode not in OUTPUT_MODES:
         raise ValueError('Unknown output mode `%s`' % output_mode)
     mode = OUTPUT_MODES[output_mode]

@@ -16,6 +16,12 @@ from .dto.intervals import ScoredInterval
 from .splitters import _fusion
 
 
+def _step_penalties(step):
+    """the penalty spec a regularised 'rounds' / 'window' step carries after its arguments (_fusion), or None"""
+    n = 6 if step[0] == 'rounds' else 5
+    return step[n] if len(step) > n else None
+
+
 def _run_device_pipeline(eng, plan, first=None):
     """Run the device steps of a pipeline plan on the loaded batch.  Returns (score or None, splits).
     first: result of the first step's first round when the load already ran it (Engine.load_and_round)."""
@@ -24,14 +30,14 @@ def _run_device_pipeline(eng, plan, first=None):
         if k == 0 and first is not None and step[0] == 'window':
             continue
         if step[0] == 'rounds':
-            _, factory, size, shift, constraint, num_rounds = step
-            eng.use_scorer(factory)
+            _, factory, size, shift, constraint, num_rounds = step[:6]
+            eng.use_scorer(factory, _step_penalties(step))
             sizes, final, _ = eng.rounds(size, shift, constraint, num_rounds, first=first if k == 0 else None)
             from .splitters.round_reducer import _log_rounds
             _log_rounds(sizes, final)
         else:
-            _, factory, size, shift, constraint = step
-            eng.use_scorer(factory)
+            _, factory, size, shift, constraint = step[:5]
+            eng.use_scorer(factory, _step_penalties(step))
             eng.round(size, shift, constraint)
     eng.use_scorer(plan['factory'])
     if plan['final'] == 'exact':
@@ -61,7 +67,7 @@ def segment_on_device(counts, plan, want_lmm=True):
             and not os.environ.get('PASIO_B200_NO_FUSED_LOAD')):      # (switch for A/B measurements)
         # the first round always starts from all positions: run it while the counts are still going up
         _, factory, size, shift, constraint = steps[0][:5]
-        eng.use_scorer(factory)
+        eng.use_scorer(factory, _step_penalties(steps[0]))
         first = eng.load_and_round(counts, size, shift, constraint, want_logfac=want_lmm)
         if want_lmm:
             eng.logfac_prefetch()                 # the sequential log-factorial sums run beside the remaining rounds
@@ -76,7 +82,7 @@ def segment_on_device(counts, plan, want_lmm=True):
 def segments_with_scores(profile, splitter):
     logger.info('Starting splitting profile of length %d' % len(profile))
     counts = np.array(profile)
-    plan = _fusion.pipeline_plan(splitter)
+    plan = _fusion.device_plan(splitter)
     if plan is not None:
         score, splits, means, lmm, sum_logfac = segment_on_device(counts, plan)
     else:

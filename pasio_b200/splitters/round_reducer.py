@@ -22,9 +22,9 @@ class RoundReducer(object):
         # (a candidate list without both ends is legal in the reference -- 0 and len(counts) are simply added to the
         # result -- but not for the fused device loop: those lists take the object route below)
         if plan is not None and isinstance(counts, np.ndarray) and _has_both_ends(split_candidates, counts):
-            factory, size, shift, constraint, num_rounds = plan
+            factory, size, shift, constraint, num_rounds = plan[:5]
             eng = _native.engine()
-            eng.use_scorer(factory)
+            eng.use_scorer(factory, plan[5] if len(plan) > 5 else None)
             eng.load(counts)
             _set_candidates(eng, counts, split_candidates)
             sizes, final, _ = eng.rounds(size, shift, constraint, num_rounds)

@@ -29,9 +29,9 @@ class SlidingWindowReducer(object):
         # (a candidate list without both ends is legal in the reference -- 0 and len(counts) are simply added to the
         # result -- but not for the fused device loop: those lists take the object route below)
         if plan is not None and isinstance(counts, np.ndarray) and _has_both_ends(split_candidates, counts):
-            factory, size, shift, constraint = plan
+            factory, size, shift, constraint = plan[:4]
             eng = _native.engine()
-            eng.use_scorer(factory)
+            eng.use_scorer(factory, plan[4] if len(plan) > 4 else None)
             eng.load(counts)
             _set_candidates(eng, counts, split_candidates)
             n_in, n_out, _ = eng.round(size, shift, constraint)

@@ -26,6 +26,39 @@ def _revlog(x):
     return 1 / np.log(x + 1)
 
 
+def penalty_spec(splitter):
+    """(length multiplier, length function, split-number multiplier, split-number function) of a regularised
+    SquareSplitter whose penalty functions are the two the reference's CLI offers (identity and 1/log(1+l),
+    default_splitters.py:36-39) -- those are element-wise, so their values can be tabulated; None otherwise (an
+    arbitrary callable keeps the host route)."""
+    builtin = (_identity, _revlog)
+    if not splitter.is_regularized:
+        return None
+    if splitter.length_regularization_function not in builtin or splitter.split_number_regularization_function not in builtin:
+        return None
+    return (splitter.length_regularization_multiplier, splitter.length_regularization_function,
+            splitter.split_number_regularization_multiplier, splitter.split_number_regularization_function)
+
+
+def penalty_tables(spec, n_length, n_split_number):
+    """Tables of the device DPs for a penalty_spec, evaluated with the reference's own expressions
+    (square_splitter.py:46-54), element by element the doubles the reference subtracts:
+    length_penalty[len] = multiplier * function(len) for len < n_length, split_number_penalty[k] = multiplier *
+    function(k + 1) for k < n_split_number (num_splits is a float array, :40), first_column_refund = multiplier * function(1).
+    -> (length_penalty or None, split_number_penalty or None, first_column_refund)"""
+    len_mult, len_fn, num_mult, num_fn = spec
+    length_penalty = split_number_penalty = None
+    refund = 0.0
+    with np.errstate(all='ignore'):
+        if len_mult != 0:
+            length_penalty = np.asarray(len_mult * len_fn(np.arange(n_length)), dtype=np.float64)
+        if num_mult != 0:
+            num_splits = np.arange(n_split_number, dtype=np.float64)
+            split_number_penalty = np.asarray(num_mult * num_fn(num_splits + 1), dtype=np.float64)
+            refund = float(num_mult * num_fn(1))
+    return length_penalty, split_number_penalty, refund
+
+
 class SquareSplitter(object):
     def __init__(self, scorer_factory,
                  length_regularization_multiplier=0,
@@ -68,28 +101,12 @@ class SquareSplitter(object):
 
     def _device_penalty_tables(self, score_computer, counts, split_candidates):
         """Penalty tables for the device version of the regularised DP, or None when it does not apply: the scorer must be
-        a pasio_b200 LogML computer and the penalty functions the two the reference's CLI offers (identity and 1/log(1+l),
-        default_splitters.py:36-39) -- an arbitrary callable need not be element-wise, so it keeps the host route.
-        The tables are evaluated with the reference's own expressions (square_splitter.py:46-54)."""
-        if not isinstance(score_computer, LogMarginalLikelyhoodComputer):
+        a pasio_b200 LogML computer and the penalty functions the two the reference's CLI offers (penalty_spec)."""
+        spec = penalty_spec(self)
+        if spec is None or not isinstance(score_computer, LogMarginalLikelyhoodComputer):
             return None
-        builtin = (_identity, _revlog)
-        if self.length_regularization_function not in builtin or self.split_number_regularization_function not in builtin:
-            return None
-        length_penalty = split_number_penalty = None
-        refund = 0.0
-        with np.errstate(all='ignore'):
-            if self.length_regularization_multiplier != 0:
-                lengths = np.arange(len(counts) + 1)                   # split_candidates[j] - split_candidates[:j] takes these values
-                length_penalty = np.asarray(self.length_regularization_multiplier * self.length_regularization_function(lengths),
-                                            dtype=np.float64)
-            if self.split_number_regularization_multiplier != 0:
-                num_splits = np.arange(len(split_candidates), dtype=np.float64)      # num_splits is a float array (:40)
-                split_number_penalty = np.asarray(
-                    self.split_number_regularization_multiplier * self.split_number_regularization_function(num_splits + 1),
-                    dtype=np.float64)
-                refund = float(self.split_number_regularization_multiplier * self.split_number_regularization_function(1))
-        return length_penalty, split_number_penalty, refund
+        # split_candidates[j] - split_candidates[:j] takes the values 0 .. len(counts); num_splits < len(split_candidates)
+        return penalty_tables(spec, len(counts) + 1, len(split_candidates))
 
     def _scorer_protocol_dp(self, score_computer, split_candidates, regularized):
         """Row-by-row recurrence through an arbitrary scorer object.
