@@ -496,22 +496,30 @@ class Engine(object):
             return np.float64(score.value), out, P, prev
         return np.float64(score.value), out
 
-    def square_split_regularized(self, length_penalty=None, split_number_penalty=None, first_column_refund=0.0):
-        """split_with_normalizations over the current candidates on the device; penalty tables as in include/pasio_b200.h"""
+    def square_split_regularized(self, length_penalty=None, split_number_penalty=None, first_column_refund=0.0,
+                                 want_arrays=False):
+        """split_with_normalizations over the current candidates on the device; penalty tables as in include/pasio_b200.h.
+        want_arrays: also return the prefix scores P and the arg-maxes prev, as square_split does."""
         self._check_exact_limits()
         m = self.candidate_count()
         splits = np.empty(m, dtype=np.int64)
         n_splits, score = _i64(0), ctypes.c_double(0.0)
         lp = None if length_penalty is None else np.ascontiguousarray(length_penalty, dtype=np.float64)
         sp = None if split_number_penalty is None else np.ascontiguousarray(split_number_penalty, dtype=np.float64)
+        P = np.empty(m) if want_arrays else None
+        prev = np.empty(m, dtype=np.int64) if want_arrays else None
         self._cands_obj = None
         self._retry(lambda: self.lib.pasio_square_split_regularized(
             self.ctx, None if lp is None else _ptr(lp, ctypes.c_double), 0 if lp is None else len(lp),
             None if sp is None else _ptr(sp, ctypes.c_double), 0 if sp is None else len(sp), float(first_column_refund),
-            _ptr(splits, ctypes.c_int64), m, ctypes.byref(n_splits), ctypes.byref(score), None, None))
+            _ptr(splits, ctypes.c_int64), m, ctypes.byref(n_splits), ctypes.byref(score),
+            _ptr(P, ctypes.c_double) if want_arrays else None,
+            _ptr(prev, ctypes.c_int64) if want_arrays else None))
         out = splits[:n_splits.value].copy()
         self._cands_obj = out
         self._cands_print = self._fingerprint(out)
+        if want_arrays:
+            return np.float64(score.value), out, P, prev
         return np.float64(score.value), out
 
     def suffix_scores(self, stop):

@@ -100,6 +100,16 @@ scatter_bits(const uint32_t *__restrict__ bits, i64 nwords, const int *__restric
     }
 }
 
+// every contig boundary survives (sliding_window_reducer.py:22 starts the union from {0, len(counts)}): a window shift
+// larger than the window size leaves candidates, the last one among them, in no window
+__global__ void mark_boundaries_kernel(const int32_t *__restrict__ bounds, i64 nb, uint32_t *keepbits)
+{
+    i64 c = (i64)blockIdx.x * blockDim.x + threadIdx.x;
+    if (c >= nb) return;
+    const int32_t b = bounds[c];
+    atomicOr(keepbits + (b >> 5), 1u << (b & 31));
+}
+
 // index of every contig boundary in the (sorted) candidate list
 __global__ void boundary_ranks_kernel(const int32_t *__restrict__ cand, i64 m,
                                       const int32_t *__restrict__ bounds, i64 nb, int32_t *__restrict__ brank)
@@ -245,7 +255,9 @@ int launch_compact_keepbits(pasio_ctx *ctx, int slot, i64 *h_count)
     int *bs = ctx->blocksum.as<int>();
     i64 *d_total = ctx->scalars.as<i64>() + 4;
     {
-        TimingScope ts(ctx, TF_COMPACT, 3);
+        TimingScope ts(ctx, TF_COMPACT, 4);
+        const i64 nb = ctx->n_contigs + 1;
+        mark_boundaries_kernel<<<(unsigned)((nb + 255) / 256), 256, 0, ctx->stream>>>(ctx->bounds.as<int32_t>(), nb, ctx->keepbits.as<uint32_t>());
         popc_block_sums<<<(unsigned)nblocks, CP_THREADS, 0, ctx->stream>>>(bits, nwords, bs);
         scan_block_sums<<<1, CP_THREADS, 0, ctx->stream>>>(bs, nblocks, d_total);
         scatter_bits<<<(unsigned)nblocks, CP_THREADS, 0, ctx->stream>>>(bits, nwords, bs, d_out, ctx->cg.as<i64>(), ctx->candC[slot].as<i64>());

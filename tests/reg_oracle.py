@@ -118,6 +118,26 @@ class FlatOracleReg(c_oracle.FlatOracle):
         super(FlatOracleReg, self).__init__(counts, alpha, beta, threads=threads)
         self.spec = spec
 
+    def square_split(self, cands):
+        """The regularised DP over one whole candidate list (dp_oracle_reg); returns (score, splits, P, prev, ns)."""
+        cands = np.ascontiguousarray(cands, dtype=np.int64)
+        C = np.ascontiguousarray(self.Cg[cands])
+        N = len(cands)
+        span = int(cands[-1] - cands[0])
+        a_int = int(self.alpha) if self.int_alpha else 0
+        self._ensure_tables(span + 1, int(C[-1] - C[0]) + a_int + 1)
+        lr, nr, refund = penalty_tables(self.spec, span + 1, N)
+        P = np.empty(N)
+        prev = np.empty(N, dtype=np.int64)
+        ns = np.empty(N, dtype=np.int64)
+        rc = lib().dp_oracle_reg(
+            _p(C, ctypes.c_int64), _p(cands, ctypes.c_int64), N, _p(self.g, ctypes.c_double), len(self.g),
+            _p(self.lg, ctypes.c_double), len(self.lg), int(self.int_alpha), float(self.alpha), self.pen,
+            _p(nr, ctypes.c_double), 0 if nr is None else len(nr), refund, _p(lr, ctypes.c_double),
+            0 if lr is None else len(lr), _p(P, ctypes.c_double), _p(prev, ctypes.c_int64), _p(ns, ctypes.c_int64))
+        assert rc == 0, rc
+        return P[-1], cands[po.backtrace(prev)], P, prev, ns
+
     def round(self, cands, window_size, window_shift, constraint):
         cands = np.ascontiguousarray(cands, dtype=np.int64)
         m = len(cands)

@@ -103,6 +103,35 @@ def test_c_round_equals_numpy_round(case, constraint, alpha):
             cands = want
 
 
+@pytest.mark.parametrize('case', PENALTY_CASES)
+@pytest.mark.parametrize('alpha', [1, 2.5])
+def test_c_square_split_equals_numpy(case, alpha):
+    """FlatOracleReg.square_split (the whole-list regularised DP of tests/reg_oracle.c): score and splits equal
+    po.square_split_regularized, and every row of its P / prev / split numbers is the numpy row recomputed from the
+    oracle's own earlier rows (so by induction the whole arrays are the numpy recurrence's)"""
+    num, length, fn = case
+    pen = ro.penalty_kwargs(num, length, fn)
+    tables = po.Tables(po.normalise_alpha(alpha), 1.0)
+    for name, counts in _contigs():
+        counts = counts[:400]
+        for cands in [np.arange(len(counts) + 1), np.concatenate([[0], np.arange(3, len(counts), 4), [len(counts)]])]:
+            score, splits, P, prev, ns = ro.FlatOracleReg(counts, alpha, 1.0, _spec(*case)).square_split(cands)
+            o_score, o_splits = po.square_split_regularized(counts, cands, tables, **pen)
+            assert score == o_score and np.array_equal(splits, o_splits), (name, case, alpha)
+            sc = po.Scorer(counts, cands, tables)
+            assert P[0] == 0 and prev[0] == 0 and ns[0] == 0
+            for j in range(1, len(cands)):
+                t = sc.row(j)
+                t += P[:j]
+                if num != 0:
+                    t -= pen['num_mult'] * pen['num_fn'](ns[:j].astype(np.float64) + 1)
+                    t[0] += pen['num_mult'] * pen['num_fn'](1)
+                if length != 0:
+                    t -= (pen['len_mult'] * pen['len_fn'](cands[j] - cands[:j]))[:j]
+                k = np.argmax(t)
+                assert prev[j] == k and P[j] == t[k] + sc.pen and ns[j] == (ns[k] + 1 if k else 0), (name, case, alpha, j)
+
+
 def test_c_rounds_multithreaded_and_pipeline_match_numpy():
     counts = synth.dnase_like(3000, 8, hotspot_share=0.3)
     spec = _spec(2.0, 5.0, 'revlog')
