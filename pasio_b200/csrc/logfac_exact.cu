@@ -353,11 +353,18 @@ int launch_logfac_at_candidates_exact(pasio_ctx *ctx, double *d_out)
     return PASIO_OK;
 }
 
-// the contig total (logfac_cumsum[-1]) of a single-contig context
+// the contig total (logfac_cumsum[-1]) of a single-contig context; of a batch, the last contig's total, which is 0 when
+// that contig has no non-zero term (the last kept term then belongs to an earlier contig)
 int logfac_exact_total(pasio_ctx *ctx, double *h_out)
 {
     *h_out = 0.0;
     if (ctx->lx_terms == 0) return PASIO_OK;
+    if (ctx->n_contigs > 1) {
+        i64 first = 0;
+        CUDA_TRY(ctx, cudaMemcpyAsync(&first, ctx->lxFirst.as<i64>() + (ctx->n_contigs - 1), 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+        if (first == ctx->lx_terms) return PASIO_OK;
+    }
     CUDA_TRY(ctx, cudaMemcpyAsync(h_out, ctx->lxSum.as<double>() + (ctx->lx_terms - 1), 8, cudaMemcpyDeviceToHost, ctx->stream));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     return PASIO_OK;
