@@ -72,7 +72,10 @@ enum { PASIO_TUNE_WINDOW_PRUNE = 0,   /* 1: window DP bounds far columns (defaul
        PASIO_TUNE_EXACT_NBLOCK = 9,   /* the exact DP hands the first n column blocks in front of the far columns (blocks b - lag + 1 ..
                                          of row block b) to worker CTAs, which evaluate them exhaustively; the diagonal sweeps the
                                          remaining lag - n blocks itself.  0 .. lag - 2, default 3 (with lag 5: a band of two blocks) */
-       PASIO_TUNE_COUNT = 10 };
+       PASIO_TUNE_WINDOW_CERTIFY = 10, /* 1 (default): in rounds after one that removed under 1 % of its candidates, window DP first
+                                         checks every large window for "every candidate survives" in one parallel pass and resumes
+                                         the ordinary pipeline at the first block that fails; 2: in every round; 0: never */
+       PASIO_TUNE_COUNT = 11 };
 
 /* ---- context ------------------------------------------------------------------------ */
 int pasio_ctx_create(int device, pasio_ctx **out);
@@ -152,6 +155,9 @@ int pasio_round(pasio_ctx *ctx, int64_t window_size, int64_t window_shift, int c
  * with the exact far-column bound (csrc/window_dp.cu) instead of evaluating them.  After
  * pasio_square_split: the same two numbers for the whole-contig DP. */
 int pasio_round_stats(const pasio_ctx *ctx, int64_t *cells, int64_t *cells_skipped);
+/* Of the most recent pasio_round (PASIO_TUNE_WINDOW_CERTIFY): windows in which every candidate was proven a survivor
+ * up front, windows whose check failed, and the rows those failed checks still proved (summed; the DP resumed after them). */
+int pasio_round_certify_stats(const pasio_ctx *ctx, int64_t *passed, int64_t *fell_back, int64_t *resume_rows_sum);
 /* The task list of the exact DP's worker CTAs (host only, no context, nothing is launched): for a candidate list of
  * n_candidates entries, lag and nblock as in PASIO_TUNE_EXACT_LAG / PASIO_TUNE_EXACT_NBLOCK, the tasks in the order the
  * worker CTAs pull them, as (row block, kind, slice) triples -- kind 0: S (self scores of the block, slice = quarter),

@@ -19,7 +19,7 @@ TAB_LOG, TAB_LGAMMA, TAB_LGAMMA_ALPHA = 0, 1, 2
 CONSTRAINTS = {'none': 0, 'zeros': 1, 'constants': 2}
 TUNE = {'window_prune': 0, 'window_phases': 1, 'exact_prune': 2, 'exact_lag': 3, 'exact_ring': 4, 'logfac_exact': 5,
         'window_speculate': 6, 'upload_narrow': 7,
-        'logfac_eager': 8, 'exact_nblock': 9}
+        'logfac_eager': 8, 'exact_nblock': 9, 'window_certify': 10}
 TIMING_FAMILIES = ['scan', 'window_dp', 'compact', 'exact_dp', 'score', 'h2d', 'd2h']
 
 _i64 = ctypes.c_int64
@@ -48,6 +48,7 @@ SIGNATURES = {
     'pasio_filter_candidates': (ctypes.c_int, [_vp, ctypes.c_int, _i64p, _i64p]),
     'pasio_round': (ctypes.c_int, [_vp, _i64, _i64, ctypes.c_int, _i64p, _i64p, _i64p]),
     'pasio_round_stats': (ctypes.c_int, [_vp, _i64p, _i64p]),
+    'pasio_round_certify_stats': (ctypes.c_int, [_vp, _i64p, _i64p, _i64p]),
     'pasio_exact_task_plan': (ctypes.c_int, [_i64, ctypes.c_int, ctypes.c_int, ctypes.POINTER(ctypes.c_int32), _i64, _i64p]),
     'pasio_upload_stats': (ctypes.c_int, [_vp, _i64p]),
     'pasio_set_tuning': (ctypes.c_int, [_vp, ctypes.c_int, ctypes.c_int]),
@@ -434,6 +435,13 @@ class Engine(object):
         a, b = _i64(0), _i64(0)
         self._check(self.lib.pasio_round_stats(self.ctx, ctypes.byref(a), ctypes.byref(b)))
         return a.value, b.value
+
+    def round_certify_stats(self):
+        """(windows proven to keep every candidate, windows whose check failed, rows those checks still proved)
+        of the most recent round"""
+        a, b, c = _i64(0), _i64(0), _i64(0)
+        self._check(self.lib.pasio_round_certify_stats(self.ctx, ctypes.byref(a), ctypes.byref(b), ctypes.byref(c)))
+        return a.value, b.value, c.value
 
     def rounds(self, window_size, window_shift, constraint, num_rounds=None, first=None):
         """RoundReducer loop on the device.  Returns (sizes before each round run, final count, cells).

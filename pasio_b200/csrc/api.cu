@@ -439,13 +439,13 @@ extern "C" int pasio_ctx_create(int device, pasio_ctx **out)
         cudaEventCreateWithFlags(&ctx->ev_lx1, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&ctx->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&ctx->ev_join, cudaEventDisableTiming) != cudaSuccess ||
-        cudaMallocHost((void **)&ctx->h_scalars, 16 * sizeof(i64)) != cudaSuccess ||
-        pasio_reserve(ctx, ctx->scalars, 16 * sizeof(i64)) != PASIO_OK) {
+        cudaMallocHost((void **)&ctx->h_scalars, 20 * sizeof(i64)) != cudaSuccess ||
+        pasio_reserve(ctx, ctx->scalars, 20 * sizeof(i64)) != PASIO_OK) {
         g_create_error = "context allocation failed: " + ctx->err;
         delete ctx;
         return PASIO_E_CUDA;
     }
-    memset(ctx->h_scalars, 0, 16 * sizeof(i64));
+    memset(ctx->h_scalars, 0, 20 * sizeof(i64));
     auto env_int = [](const char *name, int dflt) { const char *v = getenv(name); return v ? atoi(v) : dflt; };
     ctx->tune[PASIO_TUNE_WINDOW_PRUNE] = env_int("PASIO_WD_PRUNE", 1);
     ctx->tune[PASIO_TUNE_WINDOW_PHASES] = env_int("PASIO_WD_PHASES", 1);
@@ -457,6 +457,7 @@ extern "C" int pasio_ctx_create(int device, pasio_ctx **out)
     ctx->tune[PASIO_TUNE_UPLOAD_NARROW] = env_int("PASIO_B200_UPLOAD_NARROW", 1);
     ctx->tune[PASIO_TUNE_LOGFAC_EAGER] = env_int("PASIO_B200_LOGFAC_EAGER", 0);
     ctx->tune[PASIO_TUNE_EXACT_NBLOCK] = env_int("PASIO_XD_NBLOCK", 3);
+    ctx->tune[PASIO_TUNE_WINDOW_CERTIFY] = env_int("PASIO_WD_CERTIFY", 1);
     if (ctx->tune[PASIO_TUNE_EXACT_LAG] < 3 || ctx->tune[PASIO_TUNE_EXACT_LAG] > 5) ctx->tune[PASIO_TUNE_EXACT_LAG] = 5;
     *out = ctx;
     return PASIO_OK;
@@ -615,6 +616,7 @@ static int finish_load(pasio_ctx *ctx, const int64_t *offsets, int64_t n_contigs
     ctx->max_count = ctx->h_scalars[2];
     ctx->have_contig = true;
     ctx->implicit_all = true;
+    ctx->prev_round_in = 0;
     ctx->m = n + 1;
     ctx->cur = 0;
     PASIO_TRY(launch_boundary_ranks(ctx));
@@ -750,6 +752,7 @@ extern "C" int pasio_contig_load_round(pasio_ctx *ctx, const int64_t *counts, in
     i64 n_tiles = 0, tile_elems = 0;
     PASIO_TRY(launch_scan_prepare(ctx, &n_tiles, &tile_elems));
     ctx->implicit_all = true;
+    ctx->prev_round_in = 0;
     ctx->m = n + 1;
     ctx->cur = 0;
     ctx->n_small = ctx->n_medium = ctx->n_large = -1;
@@ -892,9 +895,13 @@ extern "C" int pasio_contig_load_round(pasio_ctx *ctx, const int64_t *counts, in
     i64 m_new = 0;
     PASIO_TRY(launch_compact_keepbits(ctx, nxt, &m_new));
     PASIO_TRY(d2h(ctx, ctx->h_scalars + 10, ctx->scalars.as<i64>() + 10, 24));
+    PASIO_TRY(d2h(ctx, ctx->h_scalars + 16, ctx->scalars.as<i64>() + 16, 24));
     if (cells) *cells = ctx->h_scalars[10];
     ctx->last_cells = ctx->h_scalars[10];
     ctx->last_cells_skipped = ctx->h_scalars[12];
+    for (int k = 0; k < 3; ++k) ctx->last_certify[k] = ctx->h_scalars[16 + k];
+    ctx->prev_round_in = ctx->m;
+    ctx->prev_round_out = m_new;
     ctx->cur = nxt;
     ctx->implicit_all = false;
     ctx->m = m_new;
@@ -955,8 +962,10 @@ extern "C" int pasio_candidates_set(pasio_ctx *ctx, const int64_t *cands, int64_
 {
     NEED_CTX(ctx);
     if (!ctx->have_contig) return pasio_fail(ctx, PASIO_E_STATE, "no contig loaded");
+    ctx->prev_round_in = 0;
     if (!cands) {
         ctx->implicit_all = true;
+    ctx->prev_round_in = 0;
         ctx->m = ctx->n + 1;
         return refresh_boundary_ranks(ctx);
     }
@@ -980,6 +989,7 @@ extern "C" int pasio_candidates_set(pasio_ctx *ctx, const int64_t *cands, int64_
     PASIO_TRY(launch_validate_candidates(ctx, &bad));
     if (bad) {
         ctx->implicit_all = true;
+    ctx->prev_round_in = 0;
         ctx->m = ctx->n + 1;
         refresh_boundary_ranks(ctx);
         return pasio_fail(ctx, PASIO_E_CANDIDATES,
@@ -1022,6 +1032,7 @@ extern "C" int pasio_filter_candidates(pasio_ctx *ctx, int constraint, int64_t *
     if (constraint < 0 || constraint > 2) return pasio_fail(ctx, PASIO_E_ARG, "unknown constraint %d", constraint);
     if (n_in) *n_in = ctx->m;
     PASIO_TRY(launch_filter_candidates(ctx, constraint));
+    ctx->prev_round_in = 0;
     const int nxt = 1 - ctx->cur;
     PASIO_TRY(pasio_reserve(ctx, ctx->cand[nxt], (size_t)ctx->m * 4));
     i64 m_new = 0;
@@ -1103,9 +1114,13 @@ extern "C" int pasio_round(pasio_ctx *ctx, int64_t window_size, int64_t window_s
     i64 m_new = 0;
     PASIO_TRY(launch_compact_keepbits(ctx, nxt, &m_new));
     PASIO_TRY(d2h(ctx, ctx->h_scalars + 10, ctx->scalars.as<i64>() + 10, 24));
+    PASIO_TRY(d2h(ctx, ctx->h_scalars + 16, ctx->scalars.as<i64>() + 16, 24));
     if (cells) *cells = ctx->h_scalars[10];
     ctx->last_cells = ctx->h_scalars[10];
     ctx->last_cells_skipped = ctx->h_scalars[12];
+    for (int k = 0; k < 3; ++k) ctx->last_certify[k] = ctx->h_scalars[16 + k];
+    ctx->prev_round_in = ctx->m;
+    ctx->prev_round_out = m_new;
     ctx->cur = nxt;
     ctx->implicit_all = false;
     ctx->m = m_new;
@@ -1154,6 +1169,15 @@ extern "C" int pasio_round_stats(const pasio_ctx *ctx, int64_t *cells, int64_t *
     return PASIO_OK;
 }
 
+extern "C" int pasio_round_certify_stats(const pasio_ctx *ctx, int64_t *passed, int64_t *fell_back, int64_t *resume_rows_sum)
+{
+    if (!ctx) return PASIO_E_ARG;
+    if (passed) *passed = ctx->last_certify[0];
+    if (fell_back) *fell_back = ctx->last_certify[1];
+    if (resume_rows_sum) *resume_rows_sum = ctx->last_certify[2];
+    return PASIO_OK;
+}
+
 extern "C" int pasio_set_tuning(pasio_ctx *ctx, int key, int value)
 {
     if (!ctx) return PASIO_E_ARG;
@@ -1182,6 +1206,7 @@ static int finish_square_split(pasio_ctx *ctx, i64 N, int64_t *out_splits, int64
         for (i64 k = 0; k < N; ++k) previous_splits[k] = tmp[(size_t)k];
     }
     PASIO_TRY(launch_backtrace_mark(ctx, N));
+    ctx->prev_round_in = 0;
     const int nxt = 1 - ctx->cur;
     PASIO_TRY(pasio_reserve(ctx, ctx->cand[nxt], (size_t)N * 4));
     i64 m_new = 0;

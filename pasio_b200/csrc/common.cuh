@@ -109,9 +109,11 @@ struct pasio_ctx {
 
     // tuning switches (pasio_set_tuning; defaults from the PASIO_WD_* / PASIO_XD_* environment variables)
     int tune[PASIO_TUNE_COUNT];
-    i64 *h_scalars = nullptr;    // pinned, 16 entries
+    i64 *h_scalars = nullptr;    // pinned, 20 entries
 
     i64 last_cells = 0, last_cells_skipped = 0;   // of the most recent round
+    i64 last_certify[3] = {0, 0, 0};              // of the most recent round: windows passed, fell back, rows proven before falling back
+    i64 prev_round_in = 0, prev_round_out = 0;    // candidates before / after the previous round on the current candidates (0: none)
     std::vector<i64> pw_leaf_start;      // leaf boundaries of numpy's pairwise sum for pw_n elements (pasio_segment_scores_sum)
     i64 pw_n = -1;
     std::vector<double> pw_leaf_sum;

@@ -94,6 +94,8 @@ struct WinDpParams {
     int p1_stride;
     int skip_covered;           // 0: phase-2 windows neither wait nor get skipped (experiments)
     int speculate;              // CTA kernel: try block_chain_speculative first (PASIO_TUNE_WINDOW_SPECULATE)
+    int certify;                // CTA kernel: check every pruned window for "every candidate survives" first (certify_window)
+    u64 *certify_stats;         // [0] windows that passed the check, [1] windows that fell back, [2] sum of their proven rows
     int n_lg;                   // warp-per-window kernels with the log table in shared memory: entries copied
 };
 
@@ -448,6 +450,197 @@ __device__ __forceinline__ void build_coarse_record(int jb, const ColRec *sCol, 
     fit_column_record(me.C, me.L, me.P, rec, tilt_scale_c, tilt_scale_l);
 }
 
+// ---- the whole window under one hypothesis ---------------------------------------------------
+// In the later rounds most windows keep every candidate: the first maximum of every row j is column j-1.  Fixing that
+// hypothesis for the whole window up front makes every P known before any cell is looked at,
+//     P_j = (self(j-1, j) + P_{j-1}) + pen        (block_chain_speculative's operation order),
+// so the checks of all rows are independent: row j holds iff every cell i < j-1 is strictly below T_j = t_{j-1,j}
+// (a tie at a smaller column would be the first maximum).  If every row holds, by induction over the rows P and
+// prev = j-1 are what the block pipeline computes, bit for bit.  If row j* fails, the same induction proves every row
+// before j*: the pipeline resumes at the block holding j*.
+// The rows go in groups of CT_RB blocks (sT and sRowG hold one group).  Per group: (a) self(j-1, j) in parallel,
+// (b) the sequential sum by one thread, (c) the column-block records of the group and, exactly, the near columns of
+// every row (the previous block, the triangle, column 0), (d) far columns bounded per 32 x 32 rectangle (far_pass's
+// level 1, with T_j as the row value: it is exact, so no delta_path), (e) the survivors again per 4 x 8 rectangle
+// (level 2) and what survives that cell by cell.  The far levels skip rows at and past a failure already found, and a
+// group with a failure ends the check.  Returns the first failing row, N if none.
+constexpr int CT_RB = 16;
+
+template <bool AI>
+__device__ __forceinline__ int certify_window(const WinDpParams &p, int N, ColRec *sCol, CoarseRec *sCoarse, const double *sScal0,
+                                              double *sScal1, double *sT, float4 *sRowG, double *sLbAbs, int *sSkip,
+                                              unsigned short *sL1, int *sFail, int *sL1Count, double tilt_c, double tilt_l,
+                                              u64 &skipped)
+{
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int nrb = (N - 1 + DP_JB - 1) / DP_JB;            // row blocks: rows [1 + 32k, 33 + 32k)
+    if (tid == 0) { *sFail = N; *sL1Count = 0; }
+    if (tid < CT_RB) sSkip[tid] = 0;
+    for (int kg = 0; kg < nrb; kg += CT_RB) {
+        const int r0 = 1 + DP_JB * kg, r1 = min(N, r0 + DP_JB * CT_RB), kge = min(nrb, kg + CT_RB);
+        // (a)
+        for (int j = r0 + tid; j < r1; j += WD_THREADS) {
+            const int2 me = col_lc(sCol, j), bf = col_lc(sCol, j - 1);
+            sT[j - r0] = self_score<AI>(bf.y, bf.x, make_row<AI>(me.y, me.x, p.alpha_int, p.alpha), p.gtab, p.ltab);
+        }
+        __syncthreads();
+        // (b) sT becomes T_j; running max |P| (the scale of delta)
+        if (tid == 0) {
+            double P = sCol[r0 - 1].P, mx = *sScal1;
+            for (int j = r0; j < r1; ++j) {
+                const double t = __dadd_rn(sT[j - r0], P);
+                P = __dadd_rn(t, p.pen);
+                sT[j - r0] = t;
+                sCol[j].P = P;
+                mx = fmax(mx, fabs(P));
+            }
+            *sScal1 = mx;
+        }
+        __syncthreads();
+        // (c) lane = row; the near columns j-2 .. c0 by distance (rows of a warp then gather nearby table entries)
+        for (int k = kg + warp; k < kge; k += WD_WARPS) {
+            const int jb = 1 + DP_JB * k;
+            if (jb + DP_JB <= N) build_coarse_record(jb, sCol, sCoarse + k, tilt_c, tilt_l);
+            const bool valid = jb + lane < N;
+            const int j = min(jb + lane, N - 1);
+            const double T = sT[j - r0];
+            const int2 me = col_lc(sCol, j);
+            const RowConst<AI> rme = make_row<AI>(me.y, me.x, p.alpha_int, p.alpha);
+            const int c0 = k == 0 ? 0 : jb - DP_JB;
+            const int dmax = j - c0, dmax_w = __reduce_max_sync(0xffffffffu, dmax);
+            bool ok = fabs(T) < 1e30;                           // beyond float range the far bound has no row value
+            constexpr int UN = 4;
+            for (int d = 2; d <= dmax_w; d += UN) {
+                double t[UN];
+#pragma unroll
+                for (int u = 0; u < UN; ++u) {
+                    const ColRec c = sCol[max(j - d - u, 0)];
+                    t[u] = d + u <= dmax ? __dadd_rn(self_score<AI>(c.C, c.L, rme, p.gtab, p.ltab), c.P) : -INFINITY;
+                }
+#pragma unroll
+                for (int u = 0; u < UN; ++u) ok &= t[u] < T;
+            }
+            if (c0 > 0) {                                       // column 0 is in no column block
+                const ColRec c = sCol[0];
+                ok &= __dadd_rn(self_score<AI>(c.C, c.L, rme, p.gtab, p.ltab), c.P) < T;
+            }
+            if (valid && !ok) atomicMin(sFail, j);
+            sRowG[(k - kg) * 32 + lane] = make_float4((float)T, (float)me.y, (float)me.x, 0.f);
+            double ab = valid && ok ? fabs(T) : 0.0;
+#pragma unroll
+            for (int off = 16; off > 0; off >>= 1) ab = fmax(ab, __shfl_xor_sync(0xffffffffu, ab, off));
+            if (lane == 0) sLbAbs[k - kg] = ab;
+        }
+        __syncthreads();
+        const double delta = (*sScal0 + *sScal1 + fabs(p.pen) * DP_JB) * 5.684341886080802e-14;   // 2^-44, as far_delta
+        // (d) rectangles (row block k, column block cb < k-1) of the blocks before the first failure, flat over the threads
+        {
+            const int f = *sFail;
+            const int kend = min(kge, f >= N ? nrb : (f - 1) / DP_JB), k1 = max(kg, 2);
+            int ntot = 0;
+            for (int k = k1; k < kend; ++k) ntot += k - 1;
+            for (int base = 0; base < ntot; base += WD_THREADS) {
+                const int e = base + tid;
+                bool surv = false;
+                int k = k1, cb = e;
+                if (e < ntot) {
+                    while (cb >= k - 1) { cb -= k - 1; ++k; }
+                    const int jb = 1 + DP_JB * k, nrows = min(DP_JB, N - jb);
+                    const int2 rowF = col_lc(sCol, jb), rowL = col_lc(sCol, jb + nrows - 1);
+                    const CoarseRec *rec = sCoarse + cb;
+                    const int4 ends = *reinterpret_cast<const int4 *>(rec);
+                    const double a1 = rec->a, b1 = rec->b;
+                    const double ub1 = rec->mpt + tilted_box_max<AI>(rowF.y - ends.y, rowL.y - ends.x, rowF.x - ends.w, rowL.x - ends.z,
+                                                                     a1, b1, p.gtab, p.ltab, p.alpha_int, p.alpha);
+                    const double m3 = tilted_row_min(sRowG + (k - kg) * 32, 0, nrows - 1, a1, b1, sLbAbs[k - kg], rowL.y, rowL.x);
+                    surv = !(ub1 - m3 + delta < 0.0);                     // NaN keeps the rectangle
+                    if (!surv) atomicAdd(sSkip + (k - kg), PR_CB * nrows);
+                }
+                const unsigned mask = __ballot_sync(0xffffffffu, surv);
+                if (mask) {
+                    int slot = 0;
+                    if (lane == 0) slot = atomicAdd(sL1Count, __popc(mask));
+                    slot = __shfl_sync(0xffffffffu, slot, 0);
+                    if (surv) sL1[slot + __popc(mask & ((1u << lane) - 1u))] = (unsigned short)(((k - kg) << 8) | cb);
+                }
+            }
+        }
+        __syncthreads();
+        // (e) a warp per surviving rectangle: level 2 (lane = 4 rows x 8 columns), then the cells of the surviving
+        // sub-rectangles, 4 at a time (lane = row er, column ec)
+        {
+            const int nl1 = *sL1Count;
+            const int rg = lane >> 2, q = lane & 3, er = lane >> 3, ec = lane & 7;
+            for (int e = warp; e < nl1; e += WD_WARPS) {
+                const int ent = sL1[e], kl = ent >> 8, cb = ent & 255;
+                const int jb = 1 + DP_JB * (kg + kl), nrows = min(DP_JB, N - jb);
+                const int f = __shfl_sync(0xffffffffu, *reinterpret_cast<volatile int *>(sFail), 0);
+                if (f < min(jb + DP_JB, N)) continue;           // a failure in this block or before it: not needed
+                const CoarseRec *rec = sCoarse + cb;
+                const double a = rec->a, b = rec->b;
+                const int rr0 = 4 * rg, rr1 = min(rr0 + 3, nrows - 1);
+                bool surv2 = false;
+                int sk = 0;
+                if (rr0 < nrows) {
+                    const int i0 = 1 + PR_CB * cb + PR_FB * q;
+                    const int2 cF = col_lc(sCol, i0), cL = col_lc(sCol, i0 + PR_FB - 1);
+                    const int2 gF = col_lc(sCol, jb + rr0), gL = col_lc(sCol, jb + rr1);
+                    const double m2 = tilted_box_max<AI>(gF.y - cL.y, gL.y - cF.y, gF.x - cL.x, gL.x - cF.x, a, b,
+                                                         p.gtab, p.ltab, p.alpha_int, p.alpha);
+                    const double m3 = tilted_row_min(sRowG + kl * 32, rr0, rr1, a, b, sLbAbs[kl], gL.y, gL.x);
+                    surv2 = !(rec->mpt8[q] + m2 - m3 + delta < 0.0);
+                    if (!surv2) sk = PR_FB * (rr1 - rr0 + 1);
+                }
+                unsigned m = __ballot_sync(0xffffffffu, surv2);
+                int bad = N;
+                while (m) {
+                    constexpr int UX = 4;
+                    double t[UX], T[UX];
+                    int row[UX];
+#pragma unroll
+                    for (int u = 0; u < UX; ++u) {
+                        t[u] = -INFINITY;
+                        T[u] = 0.0;
+                        row[u] = N;
+                        if (m) {
+                            const int l2 = __ffs(m) - 1;
+                            m &= m - 1;
+                            const int r = 4 * (l2 >> 2) + er;
+                            if (r < nrows) {
+                                row[u] = jb + r;
+                                const int2 rl = col_lc(sCol, jb + r);
+                                const RowConst<AI> rc = make_row<AI>(rl.y, rl.x, p.alpha_int, p.alpha);
+                                const ColRec cc = sCol[1 + PR_CB * cb + PR_FB * (l2 & 3) + ec];
+                                t[u] = __dadd_rn(self_score<AI>(cc.C, cc.L, rc, p.gtab, p.ltab), cc.P);
+                                T[u] = sT[jb + r - r0];
+                            }
+                        }
+                    }
+#pragma unroll
+                    for (int u = 0; u < UX; ++u)
+                        if (row[u] < N && !(t[u] < T[u])) bad = min(bad, row[u]);
+                }
+                if (bad < N) atomicMin(sFail, bad);
+#pragma unroll
+                for (int off = 16; off > 0; off >>= 1) sk += __shfl_xor_sync(0xffffffffu, sk, off);
+                if (lane == 0 && sk) atomicAdd(sSkip + kl, sk);
+            }
+        }
+        __syncthreads();
+        const int f = *sFail;
+        if (tid == 0) {                                         // skips count for the rows that stay proven only
+            const int kf = f >= N ? nrb : (f - 1) / DP_JB;
+            for (int k = kg; k < kge; ++k) {
+                if (k < kf) skipped += (u64)sSkip[k - kg];
+                sSkip[k - kg] = 0;
+            }
+            *sL1Count = 0;
+        }
+        if (f < N) return f;
+    }
+    return N;
+}
+
 template <bool AI, int U, int RPL, bool PRUNE>
 __global__ void __launch_bounds__(WD_THREADS, 3)
 window_dp_kernel(WinDpParams p)
@@ -653,6 +846,29 @@ window_dp_kernel(WinDpParams p)
         // (with all positions as candidates -- round 1 -- most candidates are noise, the arg-max is far away and the
         // bounds cut little: plain sweeps are faster there)
         const bool pipelined = PRUNE && N > PR_MIN_N && p.cand != nullptr;
+        bool passed = false;
+        if (pipelined && p.certify) {
+            __syncthreads();                                // sScal
+            const int f = certify_window<AI>(p, N, sCol, sCoarse, sScal, sScal + 1, sFarV, reinterpret_cast<float4 *>(sTri), sPartV,
+                                             sPartA, sList, sMisc + 2, sMisc + 3, sScal[2], sScal[3], skipped);
+            passed = f >= N;
+            // resume at the block holding the failure; rows before it are final (in the first two blocks: from the start)
+            const int kf = (f - 1) / DP_JB, res = passed || kf < 2 ? 1 : 1 + DP_JB * kf;
+            for (int j = 1 + tid; j < res; j += WD_THREADS) sPrev[j] = (unsigned short)(j - 1);
+            if (warp == 0 && !passed) {                     // max |P| of the finished rows, as finish_block leaves it
+                double ab = 0.0;
+                for (int j = 1 + lane; j < res; j += 32) ab = fmax(ab, fabs(sCol[j].P));
+#pragma unroll
+                for (int off = 16; off > 0; off >>= 1) ab = fmax(ab, __shfl_xor_sync(0xffffffffu, ab, off));
+                if (lane == 0) sScal[1] = ab;
+            }
+            if (tid == 0) {
+                atomicAdd(p.certify_stats + (passed ? 0 : 1), 1ull);
+                if (res > 1) atomicAdd(p.certify_stats + 2, (u64)(res - 1));
+            }
+            jb = passed ? N : res;
+            __syncthreads();
+        }
         for (; jb < N && (!pipelined || jb < 1 + 2 * DP_JB); jb += DP_JB) {
             dp_block_step<AI, WD_WARPS, U, RPL>(jb, N, 0, sCol, sPrev, nullptr, sPartV, sPartA, sTri,
                                                 p.gtab, p.ltab, p.alpha_int, p.alpha, p.pen, -INFINITY, 0, 0);
@@ -714,10 +930,10 @@ window_dp_kernel(WinDpParams p)
         }
 
         // ---- (C) back-trace by pointer doubling, scatter survivors ----------------------------
-        for (int k = tid; k < N; k += WD_THREADS) sMark[k] = (k == N - 1);
+        for (int k = tid; k < N; k += WD_THREADS) sMark[k] = passed || k == N - 1;
         __syncthreads();
         unsigned short *ja = sPrev, *jb2 = sJump;
-        for (int reach = 1; reach < N; reach <<= 1) {
+        for (int reach = passed ? N : 1; reach < N; reach <<= 1) {
             // nodes within `reach` hops of the end are marked; ja[k] is the node 'reach' hops before k
             for (int k = tid; k < N; k += WD_THREADS)
                 if (sMark[k]) sMark[ja[k]] = 1;
@@ -959,8 +1175,12 @@ int launch_window_dp(pasio_ctx *ctx, i64 nwin, int wsize, int wshift, int constr
     p.cells_skipped = ctx->scalars.as<u64>() + 12;
     p.work_counter = ctx->scalars.as<unsigned>() + 2 * 11;   // scalars[11]
     p.w_begin = w_begin;
+    p.certify_stats = ctx->scalars.as<u64>() + 16;
     if (keep_cell_counters) CUDA_TRY(ctx, cudaMemsetAsync(ctx->scalars.as<u64>() + 11, 0, 8, ctx->stream));   // work counter only
-    else CUDA_TRY(ctx, cudaMemsetAsync(ctx->scalars.as<u64>() + 10, 0, 24, ctx->stream));
+    else {
+        CUDA_TRY(ctx, cudaMemsetAsync(ctx->scalars.as<u64>() + 10, 0, 24, ctx->stream));
+        CUDA_TRY(ctx, cudaMemsetAsync(p.certify_stats, 0, 24, ctx->stream));
+    }
     CUDA_TRY(ctx, cudaMemsetAsync(ctx->scalars.as<u64>() + 15, 0, 8, ctx->stream));    // work counters of the warp-per-window kernels
 
     // The work lists of the prepass (launch_window_prepass with classification).  The CTA-per-window kernel is
@@ -978,6 +1198,11 @@ int launch_window_dp(pasio_ctx *ctx, i64 nwin, int wsize, int wshift, int constr
     p.n_p1 = use_lists ? ctx->n_large_p1 : n_large;
     p.skip_covered = phase_env;                                       // PASIO_WD_PHASES=0 (experiments): no window is skipped
     p.speculate = ctx->tune[PASIO_TUNE_WINDOW_SPECULATE];
+    // The check pays where most windows keep every candidate.  The previous round on the same candidates predicts that:
+    // on chr1, round 2 removes 10 % and round 3 only 0.3 %, after which most windows pass (DESIGN K4).
+    const int certify_env = ctx->tune[PASIO_TUNE_WINDOW_CERTIFY];
+    p.certify = certify_env >= 2 ||
+                (certify_env == 1 && ctx->prev_round_in > 0 && (ctx->prev_round_in - ctx->prev_round_out) * 100 < ctx->prev_round_in);
     p.done_flags = ctx->win_flags.as<unsigned char>();
     p.p1_stride = wshift > 0 && wsize / wshift > 1 ? wsize / wshift : 1;
     if (!use_lists) p.skip_covered = 0;

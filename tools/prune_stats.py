@@ -11,5 +11,7 @@ for r in range(12):
     n_in, n_out, cells = eng.round(2500, 1250, 'constants')
     ms = eng.timing()['window_dp'][0]
     c, sk = eng.round_stats()
-    print('round %d: %d -> %d cands, cells %.4g, skipped %.4g (%.1f%%), window_dp %.2f ms' % (r + 1, n_in, n_out, c, sk, 100.0 * sk / max(c, 1), ms), flush=True)
+    passed, fell, rows = eng.round_certify_stats()
+    print('round %d: %d -> %d cands, cells %.4g, skipped %.4g (%.1f%%), window_dp %.2f ms, checked windows passed %d fell back %d '
+          '(rows proven before the resume %d)' % (r + 1, n_in, n_out, c, sk, 100.0 * sk / max(c, 1), ms, passed, fell, rows), flush=True)
     if n_in == n_out: break
