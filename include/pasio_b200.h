@@ -75,7 +75,10 @@ enum { PASIO_TUNE_WINDOW_PRUNE = 0,   /* 1: window DP bounds far columns (defaul
        PASIO_TUNE_WINDOW_CERTIFY = 10, /* 1 (default): in rounds after one that removed under 1 % of its candidates, window DP first
                                          checks every large window for "every candidate survives" in one parallel pass and resumes
                                          the ordinary pipeline at the first block that fails; 2: in every round; 0: never */
-       PASIO_TUNE_COUNT = 11 };
+       PASIO_TUNE_REG_EXACT = 11,     /* whole-list DP of pasio_square_split_regularized: 1 (default): one CTA for short
+                                         candidate lists, a kernel on every SM for long ones (the threshold is
+                                         REG_EXACT_MIN_CANDIDATES in csrc/api.cu); 0: always one CTA; 2: always every SM */
+       PASIO_TUNE_COUNT = 12 };
 
 /* ---- context ------------------------------------------------------------------------ */
 int pasio_ctx_create(int device, pasio_ctx **out);

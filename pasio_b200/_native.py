@@ -19,7 +19,7 @@ TAB_LOG, TAB_LGAMMA, TAB_LGAMMA_ALPHA = 0, 1, 2
 CONSTRAINTS = {'none': 0, 'zeros': 1, 'constants': 2}
 TUNE = {'window_prune': 0, 'window_phases': 1, 'exact_prune': 2, 'exact_lag': 3, 'exact_ring': 4, 'logfac_exact': 5,
         'window_speculate': 6, 'upload_narrow': 7,
-        'logfac_eager': 8, 'exact_nblock': 9, 'window_certify': 10}
+        'logfac_eager': 8, 'exact_nblock': 9, 'window_certify': 10, 'reg_exact': 11}
 TIMING_FAMILIES = ['scan', 'window_dp', 'compact', 'exact_dp', 'score', 'h2d', 'd2h']
 
 _i64 = ctypes.c_int64

@@ -458,6 +458,7 @@ extern "C" int pasio_ctx_create(int device, pasio_ctx **out)
     ctx->tune[PASIO_TUNE_LOGFAC_EAGER] = env_int("PASIO_B200_LOGFAC_EAGER", 0);
     ctx->tune[PASIO_TUNE_EXACT_NBLOCK] = env_int("PASIO_XD_NBLOCK", 3);
     ctx->tune[PASIO_TUNE_WINDOW_CERTIFY] = env_int("PASIO_WD_CERTIFY", 1);
+    ctx->tune[PASIO_TUNE_REG_EXACT] = 1;
     if (ctx->tune[PASIO_TUNE_EXACT_LAG] < 3 || ctx->tune[PASIO_TUNE_EXACT_LAG] > 5) ctx->tune[PASIO_TUNE_EXACT_LAG] = 5;
     *out = ctx;
     return PASIO_OK;
@@ -1183,6 +1184,7 @@ extern "C" int pasio_set_tuning(pasio_ctx *ctx, int key, int value)
     if (!ctx) return PASIO_E_ARG;
     if (key < 0 || key >= PASIO_TUNE_COUNT) return pasio_fail(ctx, PASIO_E_ARG, "unknown tuning key %d", key);
     if (key == PASIO_TUNE_EXACT_LAG && (value < 3 || value > 5)) return pasio_fail(ctx, PASIO_E_ARG, "exact lag must be 3, 4 or 5");
+    if (key == PASIO_TUNE_REG_EXACT && (value < 0 || value > 2)) return pasio_fail(ctx, PASIO_E_ARG, "reg_exact must be 0, 1 or 2");
     ctx->tune[key] = value;
     if (key == PASIO_TUNE_LOGFAC_EXACT) {
         if (ctx->logfac_pending) { cudaStreamSynchronize(ctx->stream_lx); ctx->logfac_pending = false; }
@@ -1237,6 +1239,11 @@ extern "C" int pasio_square_split(pasio_ctx *ctx, int64_t *out_splits, int64_t c
     return finish_square_split(ctx, N, out_splits, cap, n_splits, score, prefix_scores, previous_splits);
 }
 
+// From this many candidates on, pasio_square_split_regularized runs the DP on every SM (K9, regularized_exact.cu) instead of
+// in one CTA (K6, regularized_dp.cu).  Measured on a B200 (1000 W): K6 is 5-9 % faster at 257 candidates, K9 1.3x faster
+// at 1 025 and 2x at 2 501 (DESIGN.md, K9; profiles/r03_reg_exact_kernels.txt).
+constexpr i64 REG_EXACT_MIN_CANDIDATES = 1025;
+
 extern "C" int pasio_square_split_regularized(pasio_ctx *ctx, const double *length_penalty, int64_t n_length_penalty,
                                               const double *split_number_penalty, int64_t n_split_number_penalty,
                                               double first_column_refund, int64_t *out_splits, int64_t cap, int64_t *n_splits,
@@ -1263,7 +1270,11 @@ extern "C" int pasio_square_split_regularized(pasio_ctx *ctx, const double *leng
         PASIO_TRY(h2d(ctx, ctx->regNR.p, split_number_penalty, (size_t)N * 8));
         d_nr = ctx->regNR.as<double>();
     }
-    PASIO_TRY(launch_regularized_dp(ctx, N, d_lr, d_nr, first_column_refund));
+    const int mode = ctx->tune[PASIO_TUNE_REG_EXACT];
+    if (mode == 2 || (mode == 1 && N >= REG_EXACT_MIN_CANDIDATES))
+        PASIO_TRY(launch_regularized_exact(ctx, N, d_lr, d_nr, first_column_refund));
+    else
+        PASIO_TRY(launch_regularized_dp(ctx, N, d_lr, d_nr, first_column_refund));
     CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));      // the caller's tables were read by the copies above
     return finish_square_split(ctx, N, out_splits, cap, n_splits, score, prefix_scores, previous_splits);
 }

@@ -188,6 +188,7 @@ int window_dp_reg_max_candidates(pasio_ctx *ctx);
 int launch_exact_dp(pasio_ctx *ctx, i64 N);                   // over ctx->dpL/dpC -> dpP/dpPrev
 int launch_exact_dp_pruned(pasio_ctx *ctx, i64 N, int lag);
 int launch_regularized_dp(pasio_ctx *ctx, i64 N, const double *d_lr, const double *d_nr, double add0);   // regularized_dp.cu   // exact_pruned.cu: the same result, far columns bounded
+int launch_regularized_exact(pasio_ctx *ctx, i64 N, const double *d_lr, const double *d_nr, double add0);   // regularized_exact.cu: the same DP on every SM
 int launch_gather_candidates(pasio_ctx *ctx);                 // current candidates -> dpL/dpC (rebased)
 int launch_backtrace_mark(pasio_ctx *ctx, i64 N);             // dpPrev -> keepbits (positions on the optimal path)
 int launch_suffix_row(pasio_ctx *ctx, i64 stop, double *d_out);

@@ -14,6 +14,28 @@
 #pragma once
 #include "common.cuh"
 
+// Flags between the CTAs of a cooperatively launched pipeline (K3 exact_dp.cu, K9 regularized_exact.cu): a CTA waits
+// until *flag >= target, then reads what was published before it; publish() makes the CTA's earlier writes visible first.
+__device__ __forceinline__ int ld_flag(const int *p) { return *reinterpret_cast<const volatile int *>(p); }
+__device__ __forceinline__ void st_flag(int *p, int v) { *reinterpret_cast<volatile int *>(p) = v; }
+
+__device__ __forceinline__ void wait_at_least(const int *flag, int target)
+{
+    if (threadIdx.x == 0) {
+        while (ld_flag(flag) < target) __nanosleep(40);
+        __threadfence();
+    }
+    __syncthreads();
+}
+__device__ __forceinline__ void publish(int *flag, int value)
+{
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence();
+        st_flag(flag, value);
+    }
+}
+
 // Per-row constants.  AI = integer alpha (table index includes alpha, s is that integer);
 // real alpha: table index is the raw count, s = (alpha + C_j) - C_i in float64 with the
 // reference's two roundings.
@@ -273,6 +295,42 @@ __device__ __forceinline__ bool block_chain_speculative(int jb, int N, ColRec *s
         sPrev16[jb + lane] = (unsigned short)arg;
     }
     return true;
+}
+
+// The dependent part of a 32-row step of the whole-list regularised DP (K6 regularized_dp.cu, K9 regularized_exact.cu),
+// one warp, lane = row jb + lane.  best / arg come in as the row's (max, first arg-max) over the columns before jb, with
+// arg a column index of the list; triS / triR hold self score and length penalty of (column jb + k, row jb + lane).
+// Resolves the rows in order: the split number of row jb + k follows its arg-max a, from this warp's registers when
+// a >= jb, else from ns[] (rows already written back).  Returns the row's P (mine), split number and NR[split number].
+__device__ __forceinline__ void reg_block_chain(int jb, int rows, const int *ns, const double *nrtab, int use_num, int use_len,
+                                                double pen, const double (*triS)[33], const double (*triR)[33],
+                                                double &best_io, int &arg_io, double &mine_out, int &ns_out, double &nrv_out)
+{
+    const int lane = threadIdx.x & 31;
+    double best = best_io;          // (local copies: the compiler keeps the arg-max update branch-free)
+    int arg = arg_io;
+    double mine = 0.0, my_nrv = 0.0;
+    int my_ns = 0;
+    for (int k = 0; k < rows; ++k) {
+        const int a = __shfl_sync(0xffffffffu, arg, k);                       // previous_splits of row jb + k
+        const int from_block = __shfl_sync(0xffffffffu, my_ns, max(a - jb, 0));
+        const int nsrc = a >= jb ? from_block : ns[a];
+        const int ns_k = a != 0 ? nsrc + 1 : 0;                               // square_splitter.py:59-60
+        const double pk = __shfl_sync(0xffffffffu, __dadd_rn(best, pen), k);  // :62
+        const double nrvk = use_num ? __ldg(nrtab + ns_k) : 0.0;
+        if (lane == k) { mine = pk; my_ns = ns_k; my_nrv = nrvk; }
+        if (lane > k) {
+            double t = __dadd_rn(triS[k][lane], pk);
+            if (use_num) t = __dsub_rn(t, nrvk);
+            if (use_len) t = __dsub_rn(t, triR[k][lane]);
+            if (t > best) { best = t; arg = jb + k; }
+        }
+    }
+    best_io = best;
+    arg_io = arg;
+    mine_out = mine;
+    ns_out = my_ns;
+    nrv_out = my_nrv;
 }
 
 // One full block step: rectangle over [col0, jb), triangle, chain.  Requires col0 <= jb and

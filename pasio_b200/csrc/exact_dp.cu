@@ -57,26 +57,6 @@ struct XdParams {
     double alpha, pen;
 };
 
-__device__ __forceinline__ int ld_flag(const int *p) { return *reinterpret_cast<const volatile int *>(p); }
-__device__ __forceinline__ void st_flag(int *p, int v) { *reinterpret_cast<volatile int *>(p) = v; }
-
-__device__ __forceinline__ void wait_at_least(const int *flag, int target)
-{
-    if (threadIdx.x == 0) {
-        while (ld_flag(flag) < target) __nanosleep(40);
-        __threadfence();
-    }
-    __syncthreads();
-}
-__device__ __forceinline__ void publish(int *flag, int value)
-{
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        __threadfence();
-        st_flag(flag, value);
-    }
-}
-
 // One XR-row x ncol-column tile.  Warp w owns rows [16w, 16w+16) of the tile; a lane holds 4 of
 // them (rows 4k + lane%4, k = 0..3) and sweeps the columns of phase lane/4 (stride 8), so one gather
 // instruction spans 4 rows + 8 columns of candidates (few L1 lines) and every column record read

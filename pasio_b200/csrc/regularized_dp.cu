@@ -107,23 +107,9 @@ regularized_dp_kernel(RegParams p)
                 if (v > best) { best = v; arg = sPartA[w][lane]; }
             }
             const int rows = min(32, N - jb);
-            double mine = 0.0, my_nrv = 0.0;
-            int my_ns = 0;
-            for (int k = 0; k < rows; ++k) {
-                const int a = __shfl_sync(0xffffffffu, arg, k);                       // previous_splits of row jb + k
-                const int from_block = __shfl_sync(0xffffffffu, my_ns, max(a - jb, 0));
-                const int nsrc = a >= jb ? from_block : p.ns[a];
-                const int ns_k = a != 0 ? nsrc + 1 : 0;                               // square_splitter.py:59-60
-                const double pk = __shfl_sync(0xffffffffu, __dadd_rn(best, p.pen), k); // :62
-                const double nrvk = p.use_num ? __ldg(p.nrtab + ns_k) : 0.0;
-                if (lane == k) { mine = pk; my_ns = ns_k; my_nrv = nrvk; }
-                if (lane > k) {
-                    double t = __dadd_rn(sTriS[k][lane], pk);
-                    if (p.use_num) t = __dsub_rn(t, nrvk);
-                    if (p.use_len) t = __dsub_rn(t, sTriR[k][lane]);
-                    if (t > best) { best = t; arg = jb + k; }
-                }
-            }
+            double mine, my_nrv;
+            int my_ns;
+            reg_block_chain(jb, rows, p.ns, p.nrtab, p.use_num, p.use_len, p.pen, sTriS, sTriR, best, arg, mine, my_ns, my_nrv);
             if (lane < rows) {
                 p.P[jb + lane] = mine;
                 p.prev[jb + lane] = arg;
