@@ -205,6 +205,16 @@ int pasio_set_penalties(pasio_ctx *ctx, const double *split_number_penalty, int6
  * prefix_scores / previous_splits (optional, N entries each) expose the DP arrays. */
 int pasio_square_split(pasio_ctx *ctx, int64_t *out_splits, int64_t cap, int64_t *n_splits,
                        double *score, double *prefix_scores, int64_t *previous_splits);
+/* The same DP for every contig of a loaded batch (any n_contigs >= 1), each over its own slice of the CURRENT
+ * candidates, contigs independent of each other (the reference segments them one by one): the candidates are replaced
+ * by the union of the contigs' split points, which holds every contig boundary.  Lists of at most
+ * window_dp_max_candidates (8 192 on a B200) run together as whole-list windows of the window DP, longer lists through
+ * the whole-chip DP one after another.  n_out: the new candidate count; cells / cells_skipped: summed over all contigs,
+ * as pasio_round_stats reports them afterwards.  No score is returned (there is one per contig; pasio_segment_scores
+ * gives the parts).  Errors, all raised before anything changes: PASIO_E_TABLE_TOO_SHORT (the tables must cover the
+ * longest contig and its total count; grow them and call again), PASIO_E_TOO_LARGE (a contig's own total count + alpha
+ * reaches 2^31; the message names the contig -- the batch's sum may exceed it), PASIO_E_STATE (no contig / params). */
+int pasio_square_split_batch(pasio_ctx *ctx, int64_t *n_out, int64_t *cells, int64_t *cells_skipped);
 /* SquareSplitter.split_with_normalizations (square_splitter.py:29-65) for element-wise penalty functions: per cell
  *   t = self_score + P_i - split_number_penalty[num_splits_i] (+ first_column_refund for i = 0) - length_penalty[L_j - L_i],
  * in that order, first arg-max, num_splits_j = prev_j ? num_splits[prev_j] + 1 : 0.  The caller builds the tables with

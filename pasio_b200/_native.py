@@ -55,6 +55,7 @@ SIGNATURES = {
     'pasio_rounds': (ctypes.c_int, [_vp, _i64, _i64, ctypes.c_int, _i64, _i64p, _i64p, _i64p, _i64p, _i64]),
     'pasio_set_penalties': (ctypes.c_int, [_vp, _f64p, _i64, ctypes.c_double, _f64p, _i64]),
     'pasio_square_split': (ctypes.c_int, [_vp, _i64p, _i64, _i64p, _f64p, _f64p, _i64p]),
+    'pasio_square_split_batch': (ctypes.c_int, [_vp, _i64p, _i64p, _i64p]),
     'pasio_square_split_regularized': (ctypes.c_int, [_vp, _f64p, _i64, _f64p, _i64, ctypes.c_double, _i64p, _i64, _i64p, _f64p,
                                                      _f64p, _i64p]),
     'pasio_suffix_scores': (ctypes.c_int, [_vp, _i64, _f64p]),
@@ -106,6 +107,12 @@ def _ptr(arr, ct):
 
 class PasioDeviceError(RuntimeError):
     pass
+
+
+def exact_total_fits(total, alpha):
+    """whether the whole-list DP can take a contig of this total count: it indexes the lgamma table with count + alpha in
+    32 bits"""
+    return total + alpha < 2 ** 31 - 2
 
 
 class _PinnedPool(object):
@@ -480,7 +487,7 @@ class Engine(object):
         table up to there: refuse clearly before any multi-GB table is built.  (The default rounds pipeline has no such
         limit: its tables only reach the largest count inside one window.)"""
         n, total, _ = self.info()
-        if total + (self._params[1] if self._params else 0) >= 2 ** 31 - 2:
+        if not exact_total_fits(total, self._params[1] if self._params else 0):
             raise PasioDeviceError('pasio_b200: the exact SquareSplitter DP over a whole contig needs the total count (%d) below '
                                    '2^31; use the default `rounds` algorithm for deep-coverage contigs' % total)
 
@@ -503,6 +510,14 @@ class Engine(object):
         if want_arrays:
             return np.float64(score.value), out, P, prev
         return np.float64(score.value), out
+
+    def square_split_batch(self):
+        """square_split of every contig of the loaded batch over its own slice of the current candidates; they are
+        replaced by the union of the splits.  A contig whose own total count is too large raises PasioDeviceError."""
+        n_out, cells, skipped = _i64(0), _i64(0), _i64(0)
+        self._cands_obj = None
+        self._retry(lambda: self.lib.pasio_square_split_batch(self.ctx, ctypes.byref(n_out), ctypes.byref(cells),
+                                                              ctypes.byref(skipped)))
 
     def square_split_regularized(self, length_penalty=None, split_number_penalty=None, first_column_refund=0.0,
                                  want_arrays=False):

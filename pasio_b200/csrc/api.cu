@@ -1076,6 +1076,47 @@ static int build_window_table(pasio_ctx *ctx, i64 wsize, i64 wshift, i64 *nwin_o
     return PASIO_OK;
 }
 
+// index of contig c's first and last candidate in the current list
+static void contig_ranks(const pasio_ctx *ctx, i64 c, i64 *b0, i64 *b1)
+{
+    if (ctx->n_contigs == 1) { *b0 = 0; *b1 = ctx->m - 1; return; }
+    *b0 = ctx->h_brank[(size_t)c];
+    *b1 = ctx->h_brank[(size_t)c + 1];
+}
+
+// Window table of pasio_square_split_batch: one window [b0, b1] over the whole candidate list of every contig with at
+// most `cap` candidates, none for the longer ones.  Under constraint none such a window's DP is SquareSplitter.split of
+// that list, and its back-trace marks exactly the contig's split points.  *max_m: the most candidates of a window.
+static int build_whole_list_windows(pasio_ctx *ctx, i64 cap, i64 *nwin_out, i64 *max_m)
+{
+    *max_m = 0;
+    if (ctx->n_contigs == 1) {                                 // the closed form with size = shift = m - 1: window [0, m)
+        *nwin_out = ctx->m <= cap ? 1 : 0;
+        if (*nwin_out) *max_m = ctx->m;
+        return PASIO_OK;
+    }
+    ctx->h_win_st.clear();
+    ctx->h_win_en.clear();
+    for (i64 c = 0; c < ctx->n_contigs; ++c) {
+        i64 b0, b1;
+        contig_ranks(ctx, c, &b0, &b1);
+        if (b1 - b0 + 1 > cap) continue;
+        ctx->h_win_st.push_back((int32_t)b0);
+        ctx->h_win_en.push_back((int32_t)(b1 + 1));
+        *max_m = std::max(*max_m, b1 - b0 + 1);
+    }
+    const size_t nw = ctx->h_win_st.size();
+    if (nw) {
+        PASIO_TRY(pasio_reserve(ctx, ctx->win_st, nw * 4));
+        PASIO_TRY(pasio_reserve(ctx, ctx->win_en, nw * 4));
+        PASIO_TRY(h2d(ctx, ctx->win_st.p, ctx->h_win_st.data(), nw * 4));
+        PASIO_TRY(h2d(ctx, ctx->win_en.p, ctx->h_win_en.data(), nw * 4));
+        CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));   // host vectors are reused by the next call
+    }
+    *nwin_out = (i64)nw;
+    return PASIO_OK;
+}
+
 extern "C" int pasio_round(pasio_ctx *ctx, int64_t window_size, int64_t window_shift, int constraint,
                            int64_t *n_in, int64_t *n_out, int64_t *cells)
 {
@@ -1237,6 +1278,89 @@ extern "C" int pasio_square_split(pasio_ctx *ctx, int64_t *out_splits, int64_t c
     PASIO_TRY(launch_gather_candidates(ctx));
     PASIO_TRY(launch_exact_dp(ctx, N));
     return finish_square_split(ctx, N, out_splits, cap, n_splits, score, prefix_scores, previous_splits);
+}
+
+// SquareSplitter.split of every contig's slice of the current candidates, contigs independent of each other.  Lists that
+// fit one CTA window (window_dp_max_candidates) run together as whole-list windows of the window DP (K4); longer lists run
+// through K3 one after another, each gathered into K3's contig-local arrays and back-traced into the same survivor
+// bitmap.  pasio_round clears the bitmap before K4 and compacts it after; here the clear comes once before K4 and the
+// compaction once after the last K3 back-trace, so the splits of both classes end up in one list.
+extern "C" int pasio_square_split_batch(pasio_ctx *ctx, int64_t *n_out, int64_t *cells, int64_t *cells_skipped)
+{
+    NEED_CTX(ctx);
+    if (!ctx->have_contig) return pasio_fail(ctx, PASIO_E_STATE, "no contig loaded");
+    if (!ctx->have_params) return pasio_fail(ctx, PASIO_E_STATE, "pasio_set_params has not been called");
+    if (n_out) *n_out = ctx->m;
+    if (cells) *cells = 0;
+    if (cells_skipped) *cells_skipped = 0;
+
+    // every check before anything is written: after PASIO_E_TABLE_TOO_SHORT or PASIO_E_TOO_LARGE the state is unchanged
+    PASIO_TRY(pasio_reserve(ctx, ctx->dpJump, 3 * sizeof(i64)));
+    PASIO_TRY(launch_batch_contig_stats(ctx, ctx->dpJump.as<u64>()));
+    i64 stats[3];
+    PASIO_TRY(d2h(ctx, stats, ctx->dpJump.p, sizeof stats));
+    if (stats[2] >= 0)
+        return pasio_fail(ctx, PASIO_E_TOO_LARGE, "contig %lld of the batch: its total count does not fit the 32-bit DP index "
+                          "(the whole-list DP needs count + alpha < 2^31 per contig)", (long long)stats[2]);
+    PASIO_TRY(check_dp_tables(ctx, stats[0], stats[1]));
+
+    const i64 cap = window_dp_max_candidates(ctx);
+    i64 nwin = 0, max_short = 0, max_long = 0;
+    PASIO_TRY(build_whole_list_windows(ctx, cap, &nwin, &max_short));
+    for (i64 c = 0; c < ctx->n_contigs; ++c) {
+        i64 b0, b1;
+        contig_ranks(ctx, c, &b0, &b1);
+        if (b1 - b0 + 1 > cap) max_long = std::max(max_long, b1 - b0 + 1);
+    }
+
+    const size_t bit_bytes = (size_t)((ctx->n + 1 + 31) / 32 + 2) * 4;
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->keepbits.p, 0, bit_bytes, ctx->stream));
+    if (nwin > 0) {
+        // size = shift = the longest short list - 1: every window is phase 1 and holds its whole list (1- and 2-candidate
+        // lists included: their window keeps both ends, as the compaction's boundary marks do anyway)
+        const int wsize = (int)std::max<i64>(1, max_short - 1);
+        i64 max_span = 0, max_cnt = 0;
+        PASIO_TRY(launch_window_prepass(ctx, nwin, wsize, wsize, &max_span, &max_cnt, PASIO_CONSTRAINT_NONE));
+        PASIO_TRY(launch_window_dp(ctx, nwin, wsize, wsize, PASIO_CONSTRAINT_NONE));
+        // the cell counters are read behind the compaction's synchronisation (K3 does not touch scalars[10..12])
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_scalars + 10, ctx->scalars.as<i64>() + 10, 24, cudaMemcpyDeviceToHost, ctx->stream));
+    }
+    i64 long_cells = 0, long_skipped = 0;
+    if (max_long > 0) {
+        // sized once for the longest list (grow-only buffers; K3 grows its own scratch the same way)
+        PASIO_TRY(pasio_reserve(ctx, ctx->dpL, (size_t)max_long * 4));
+        PASIO_TRY(pasio_reserve(ctx, ctx->dpC, (size_t)max_long * 4));
+        PASIO_TRY(pasio_reserve(ctx, ctx->dpP, (size_t)max_long * 8));
+        PASIO_TRY(pasio_reserve(ctx, ctx->dpPrev, (size_t)max_long * 4));
+        PASIO_TRY(pasio_reserve(ctx, ctx->dpJump, (size_t)max_long * 8));
+        PASIO_TRY(pasio_reserve(ctx, ctx->dpMark, (size_t)max_long));
+        for (i64 c = 0; c < ctx->n_contigs; ++c) {
+            i64 b0, b1;
+            contig_ranks(ctx, c, &b0, &b1);
+            const i64 N = b1 - b0 + 1;
+            if (N <= cap) continue;
+            PASIO_TRY(launch_gather_slice(ctx, b0, N));
+            PASIO_TRY(launch_exact_dp(ctx, N));
+            long_cells += ctx->last_cells;
+            long_skipped += ctx->last_cells_skipped;
+            PASIO_TRY(launch_backtrace_mark_slice(ctx, b0, N));
+        }
+    }
+
+    const int nxt = 1 - ctx->cur;
+    PASIO_TRY(pasio_reserve(ctx, ctx->cand[nxt], (size_t)ctx->m * 4));
+    i64 m_new = 0;
+    PASIO_TRY(launch_compact_keepbits(ctx, nxt, &m_new));        // synchronises: the cell counters above have arrived
+    ctx->last_cells = long_cells + (nwin > 0 ? ctx->h_scalars[10] : 0);
+    ctx->last_cells_skipped = long_skipped + (nwin > 0 ? ctx->h_scalars[12] : 0);
+    ctx->prev_round_in = 0;
+    ctx->cur = nxt;
+    ctx->implicit_all = false;
+    ctx->m = m_new;
+    if (n_out) *n_out = m_new;
+    if (cells) *cells = ctx->last_cells;
+    if (cells_skipped) *cells_skipped = ctx->last_cells_skipped;
+    return refresh_boundary_ranks(ctx);
 }
 
 // From this many candidates on, pasio_square_split_regularized runs the DP on every SM (K9, regularized_exact.cu) instead of

@@ -193,6 +193,11 @@ int launch_gather_candidates(pasio_ctx *ctx);                 // current candida
 int launch_backtrace_mark(pasio_ctx *ctx, i64 N);             // dpPrev -> keepbits (positions on the optimal path)
 int launch_suffix_row(pasio_ctx *ctx, i64 stop, double *d_out);
 
+// exact_batch.cu: the per-contig pieces of pasio_square_split_batch
+int launch_batch_contig_stats(pasio_ctx *ctx, u64 *d_out);   // d_out[0..2]: largest span, largest total, first contig over 2^31
+int launch_gather_slice(pasio_ctx *ctx, i64 b0, i64 m);       // candidates [b0, b0 + m) -> dpL/dpC (rebased)
+int launch_backtrace_mark_slice(pasio_ctx *ctx, i64 b0, i64 N);   // dpPrev -> OR into keepbits at candidates b0 + k; no clear
+
 // score.cu
 int launch_segment_scores(pasio_ctx *ctx, double *d_scores, i64 *d_segcounts, double *d_means);
 int launch_pairwise_leaves(pasio_ctx *ctx, const double *d_values, const i64 *d_leaf_start, i64 n_leaves, double *d_leaf_sum);

@@ -279,8 +279,11 @@ def _batches(contigs, plan):
         n = int(run_len.sum())
         logger.info('Starting chrom %s of length %d' % (chrom, n))
         item = (chrom, chrom_start, run_len, run_val)
-        # the exact DP is a single-contig kernel; other splitter objects go contig by contig through their protocol
-        if plan is None or n >= BATCH_ALONE or BATCH_NT <= 0 or plan['final'] != 'nop':
+        # other splitter objects go contig by contig through their protocol; so does a contig too deep for the exact
+        # DP, which then refuses it on its own (Engine.square_split)
+        too_deep = plan is not None and plan['final'] == 'exact' and not _native.exact_total_fits(
+            int(np.dot(run_len, run_val)), plan['factory'].alpha)
+        if plan is None or n >= BATCH_ALONE or BATCH_NT <= 0 or too_deep:
             if pending:
                 yield pending
                 pending, pending_nt = [], 0

@@ -41,7 +41,10 @@ def _run_device_pipeline(eng, plan, first=None):
             eng.round(size, shift, constraint)
     eng.use_scorer(plan['factory'])
     if plan['final'] == 'exact':
-        score, _ = eng.square_split()
+        if eng.info()[2] > 1:
+            eng.square_split_batch()              # every contig's DP over its own slice; no score (one per contig)
+        else:
+            score, _ = eng.square_split()
     return score
 
 
