@@ -158,8 +158,9 @@ int pasio_round(pasio_ctx *ctx, int64_t window_size, int64_t window_shift, int c
  * with the exact far-column bound (csrc/window_dp.cu) instead of evaluating them.  After
  * pasio_square_split: the same two numbers for the whole-contig DP. */
 int pasio_round_stats(const pasio_ctx *ctx, int64_t *cells, int64_t *cells_skipped);
-/* Of the most recent pasio_round (PASIO_TUNE_WINDOW_CERTIFY): windows in which every candidate was proven a survivor
- * up front, windows whose check failed, and the rows those failed checks still proved (summed; the DP resumed after them). */
+/* Of the most recent pasio_round or pasio_square_split_batch (PASIO_TUNE_WINDOW_CERTIFY): windows in which every
+ * candidate was proven a survivor up front, windows whose check failed, and the rows those failed checks still proved
+ * (summed; the DP resumed after them). */
 int pasio_round_certify_stats(const pasio_ctx *ctx, int64_t *passed, int64_t *fell_back, int64_t *resume_rows_sum);
 /* The task list of the exact DP's worker CTAs (host only, no context, nothing is launched): for a candidate list of
  * n_candidates entries, lag and nblock as in PASIO_TUNE_EXACT_LAG / PASIO_TUNE_EXACT_NBLOCK, the tasks in the order the

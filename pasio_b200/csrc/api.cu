@@ -1322,8 +1322,10 @@ extern "C" int pasio_square_split_batch(pasio_ctx *ctx, int64_t *n_out, int64_t 
         i64 max_span = 0, max_cnt = 0;
         PASIO_TRY(launch_window_prepass(ctx, nwin, wsize, wsize, &max_span, &max_cnt, PASIO_CONSTRAINT_NONE));
         PASIO_TRY(launch_window_dp(ctx, nwin, wsize, wsize, PASIO_CONSTRAINT_NONE));
-        // the cell counters are read behind the compaction's synchronisation (K3 does not touch scalars[10..12])
+        // the cell and check counters are read behind the compaction's synchronisation (K3 does not touch scalars[10..12]
+        // or [16..18])
         CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_scalars + 10, ctx->scalars.as<i64>() + 10, 24, cudaMemcpyDeviceToHost, ctx->stream));
+        CUDA_TRY(ctx, cudaMemcpyAsync(ctx->h_scalars + 16, ctx->scalars.as<i64>() + 16, 24, cudaMemcpyDeviceToHost, ctx->stream));
     }
     i64 long_cells = 0, long_skipped = 0;
     if (max_long > 0) {
@@ -1353,6 +1355,7 @@ extern "C" int pasio_square_split_batch(pasio_ctx *ctx, int64_t *n_out, int64_t 
     PASIO_TRY(launch_compact_keepbits(ctx, nxt, &m_new));        // synchronises: the cell counters above have arrived
     ctx->last_cells = long_cells + (nwin > 0 ? ctx->h_scalars[10] : 0);
     ctx->last_cells_skipped = long_skipped + (nwin > 0 ? ctx->h_scalars[12] : 0);
+    for (int k = 0; k < 3; ++k) ctx->last_certify[k] = nwin > 0 ? ctx->h_scalars[16 + k] : 0;
     ctx->prev_round_in = 0;
     ctx->cur = nxt;
     ctx->implicit_all = false;
